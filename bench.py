@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus N --steps K ...  the CPU arm: the oracle port of the reference's path
                                                              (one process with threaded BLAS AND a train_mp.py-style pool of
                                                              forked single-threaded workers; the faster one is the value)
+    python bench.py ... --dump-outputs DIR                   also writes the last timed step's outputs as DIR/<name>.npy
 
 A step = one synchronous minibatch SGD step of the hot path over one batch of synthetic macaronic sentences:
 table build for the current theta (K2), unary products (K1), 3 sweeps of level-batched message passing
@@ -66,7 +67,14 @@ def parse():
     ap.add_argument('--sentences-per-user', type=int, default=100)
     ap.add_argument('--user-adapt', action='store_true', help='c4: every user owns a theta pair (train.py --user_adapt)')
     ap.add_argument('--traffic-file', default='r2_k4_traffic.json', help='profiles/<file>: DRAM bytes per K4 launch from the committed ncu capture')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='GPU arm: write what the last timed step returned as DIR/<name>.npy (float64), to compare two builds on '
+                         'the same seeded inputs')
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if a.dump_outputs and a.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of the GPU arm (--impl ours)')
     if a.config == 'c5':                                             # run-predictions.sh:12 at the size BASELINE names
         d = ap.parse_args([])
         if a.V == d.V: a.V = 50000
@@ -433,7 +441,18 @@ class Workload(object):
         self.peaked.append(float(h[15]))
         self.all_peaked.append(float(h[15]))
         self.thetas.append([round(float(x), 3) for x in list(self.tr.theta_ee) + list(self.tr.theta_ed)])
+        self.last = h
         return h
+
+    def outputs(self):
+        """What the last step handed its caller: the reduced 16-vector (Trainer.step) and, when training, theta after the update
+        (theta_ee then theta_ed) and, with per-user theta, this rank's users' theta in user order."""
+        out = {'reduced': self.last}
+        if self.train:
+            out['theta'] = np.concatenate([self.tr.theta_ee, self.tr.theta_ed])
+        if self.corpus is None:
+            out['user_theta'] = np.array([np.concatenate(self.tr.domain2theta[u]) for u in self.mine])
+        return {k: np.array(v, dtype=np.float64) for k, v in out.items()}
 
     def step(self):
         if self.corpus is None:                                             # c4 --user-adapt: one engine pass per user
@@ -517,6 +536,10 @@ def ours(a):
     tm1 = (eng.plan_template_hits, eng.plan_template_misses)
     peaked_value = list(w.peaked)
     value = w.n_global * a.steps / (ms / 1e3)
+    if a.dump_outputs and rank == 0:                          # before the e2e and profiling steps move theta on
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, x in w.outputs().items():
+            np.save(os.path.join(a.dump_outputs, name + '.npy'), x)
 
     # ---- e2e: host sentence arrays in, reduced gradient out, every step
     e2e = None

@@ -7,6 +7,7 @@ import sys
 import time
 from contextlib import redirect_stdout
 
+import numpy as np
 import pytest
 import torch
 
@@ -29,23 +30,29 @@ class _Event(object):
         return max((other.t - self.t) * 1e3, 1e-3)
 
 
-@pytest.mark.parametrize('extra', [[], ['--config', 'c4', '--users', '3', '--sentences-per-user', '4'],
-                                   ['--config', 'c4', '--users', '3', '--sentences-per-user', '4', '--user-adapt'],
-                                   ['--config', 'c5', '--V', '96', '--sweeps', '4'], ['--scaling', 'strong', '--msg-passes', '3']],
-                         ids=['c3', 'c4', 'c4_adapt', 'c5', 'c3_strong'])
-def test_bench_gpu_arm_dry_run(monkeypatch, extra):
+CONFIGS = {'c3': [], 'c4': ['--config', 'c4', '--users', '3', '--sentences-per-user', '4'],
+           'c4_adapt': ['--config', 'c4', '--users', '3', '--sentences-per-user', '4', '--user-adapt'],
+           'c5': ['--config', 'c5', '--V', '96', '--sweeps', '4'], 'c3_strong': ['--scaling', 'strong', '--msg-passes', '3']}
+
+
+def dry_run(monkeypatch, extra, steps=2, warmup=1):
     monkeypatch.setattr(engine, 'Kernels', FakeKernels)
     monkeypatch.setattr(torch.cuda, 'set_device', lambda *_: None)
     monkeypatch.setattr(torch.cuda, 'synchronize', lambda *_: None)
     monkeypatch.setattr(torch.cuda, 'Event', _Event)
     real_tensor = torch.tensor
     monkeypatch.setattr(torch, 'tensor', lambda *a, **k: real_tensor(*a, **{x: y for x, y in k.items() if x != 'device'}))
-    monkeypatch.setattr(sys, 'argv', ['bench.py', '--steps', '2', '--warmup', '1', '--sentences', '6', '--V', '96', '--Vd', '12', '--k', '4',
-                                      '--no-cpu-baseline'] + extra)
+    monkeypatch.setattr(sys, 'argv', ['bench.py', '--steps', str(steps), '--warmup', str(warmup), '--sentences', '6', '--V', '96',
+                                      '--Vd', '12', '--k', '4', '--no-cpu-baseline'] + extra)
     buf = io.StringIO()
     with redirect_stdout(buf):
         bench.ours(bench.parse())
-    line = json.loads(buf.getvalue().strip().splitlines()[-1])
+    return json.loads(buf.getvalue().strip().splitlines()[-1])
+
+
+@pytest.mark.parametrize('extra', list(CONFIGS.values()), ids=list(CONFIGS))
+def test_bench_gpu_arm_dry_run(monkeypatch, extra):
+    line = dry_run(monkeypatch, extra)
     for key in ('metric', 'value', 'unit', 'n_gpus', 'steps', 'warmup', 'ms_per_step', 'higher_is_better', 'scaling', 'vs_baseline',
                 'dtype', 'data', 'config', 'clocks', 'e2e', 'gpu_launches', 'roofline', 'hbm_kernels', 'cpu_baseline', 'host',
                 'message_rows'):
@@ -55,3 +62,39 @@ def test_bench_gpu_arm_dry_run(monkeypatch, extra):
     assert set(line['roofline']) >= {'bound', 'achieved', 'peak', 'unit', 'frac', 'traffic', 'by_passes'}
     assert line['scaling'] == ('strong' if ('c4' in extra or 'strong' in extra) else 'weak')
     assert 'workload' in line['config']
+
+
+@pytest.mark.parametrize('name', ['c3', 'c4_adapt', 'c5'])
+def test_bench_dump_outputs_are_the_last_timed_step(monkeypatch, tmp_path, name):
+    """--dump-outputs writes, as float64, what the last of exactly --steps timed steps returned; a second run with the same
+    arguments sees the same inputs and writes the same arrays"""
+    steps, warmup = 3, 2
+    finish, seen = bench.Workload._finish, []
+
+    def record(self, red):
+        seen.append(np.array(finish(self, red)))
+        return seen[-1]
+    monkeypatch.setattr(bench.Workload, '_finish', record)
+    runs = []
+    for i in range(2):
+        del seen[:]
+        line = dry_run(monkeypatch, CONFIGS[name] + ['--dump-outputs', str(tmp_path / str(i))], steps=steps, warmup=warmup)
+        runs.append({p.stem: np.load(p) for p in (tmp_path / str(i)).iterdir()})
+        assert len(line['message_rows']['ranks_switched_to_three_passes_per_step']) == steps
+        np.testing.assert_array_equal(runs[-1]['reduced'], seen[warmup + steps - 1])
+    want = {'c3': {'reduced', 'theta'}, 'c4_adapt': {'reduced', 'theta', 'user_theta'}, 'c5': {'reduced'}}[name]
+    assert set(runs[0]) == want
+    for k in want:
+        assert runs[0][k].dtype == np.float64
+        np.testing.assert_array_equal(runs[0][k], runs[1][k])
+    assert runs[0]['reduced'].shape == (16,) and runs[0]['reduced'][14] == (12 if name == 'c4_adapt' else 6)
+    if 'theta' in want:
+        np.testing.assert_allclose(runs[0]['theta'], line['message_rows']['theta_after_each_step'][warmup + steps - 1], atol=6e-4)
+    if name == 'c4_adapt':
+        assert runs[0]['user_theta'].shape == (3, 9)
+
+
+def test_bench_rejects_zero_steps(monkeypatch):
+    monkeypatch.setattr(sys, 'argv', ['bench.py', '--steps', '0'])
+    with pytest.raises(SystemExit):
+        bench.parse()

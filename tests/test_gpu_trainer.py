@@ -57,15 +57,18 @@ def test_batch_sgd_many_returns_reference_result_lists():
     assert res[0][2].shape == (1, 3) and res[0][3].shape == (1, 6)
 
 
-def test_bench_line_small():
+def test_bench_line_small(tmp_path):
     out = subprocess.run([sys.executable, os.path.join(REPO, 'bench.py'), '--steps', '1', '--warmup', '1', '--sentences',
-                          '16', '--V', '1024', '--Vd', '128', '--k', '6', '--cpu-sample', '2'], capture_output=True,
-                         text=True, timeout=600)
+                          '16', '--V', '1024', '--Vd', '128', '--k', '6', '--cpu-sample', '2', '--dump-outputs', str(tmp_path)],
+                         capture_output=True, text=True, timeout=600)
     assert out.returncode == 0, out.stderr[-2000:]
     line = json.loads(out.stdout.strip().splitlines()[-1])
     for key in ('metric', 'value', 'unit', 'n_gpus', 'ms_per_step', 'clocks', 'e2e', 'gpu_launches', 'roofline', 'cpu_baseline'):
         assert key in line
     assert line['gpu_launches'] > 0 and line['value'] > 0 and line['e2e']['value'] > 0
+    red, theta = np.load(tmp_path / 'reduced.npy'), np.load(tmp_path / 'theta.npy')
+    assert red.shape == (16,) and red[14] == 16 and np.isfinite(red).all()
+    np.testing.assert_allclose(theta, line['message_rows']['theta_after_each_step'][1], atol=6e-4)   # the second step: the timed one
 
 
 def test_adapt_trainer_batched_domains_vs_oracle():

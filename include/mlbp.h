@@ -172,6 +172,16 @@ int mlbp_spike_correct(const int32_t *spike_words, const int32_t *spike_cnt, con
  *   more entries equal to the K-th value than were listed): NumPy's order among exactly equal values is an implementation
  *   detail, so a caller that has to reproduce it falls back to the host calls for that row.  1 <= K <= min(V, 1024).       */
 int mlbp_topk_rows(const float *X, int ldx, int V, int n_rows, int K, int32_t *idx, float *val, int32_t *n_ties, void *stream);
+/* K7.  The .dist text of n_rows belief rows (FactorGraph.to_dist, LBP.py:125-143), on the device: row r of X (fp32, row stride
+ *   ldx, V entries) becomes the bytes of  ' '.join('%0.6f' % x for x in np.log(row.astype(np.float64)))  at
+ *   out[offsets[r] .. offsets[r + 1]), offsets[0] = 0 (int64, n_rows + 1 entries); no separator after a row's last number.
+ *   The log is the correctly rounded float64 log of each input and the decimals are CPython's (round half to even on the exact
+ *   binary value): 0 -> "-inf", NaN or x < 0 -> "nan", +inf -> "inf", a negative value that rounds to zero -> "-0.000000".
+ *   out_bytes (the capacity of out) must be at least MLBP_FMT_MAX_BYTES * V * n_rows: checked on the host, nothing is launched
+ *   otherwise.  Deterministic.  n_rows = 0 only writes offsets[0].                                                      */
+#define MLBP_FMT_MAX_BYTES   12   /* "-103.278930" (log of the smallest subnormal) plus its separator                 */
+int mlbp_format_log_rows(const float *X, int ldx, int V, int n_rows, char *out, int64_t out_bytes, int64_t *offsets,
+                         void *stream);
 /* Approximate paths (use_approx_inference LBP.py:506-507, :515-516 -> au.sparse_vec_mat_dot pyx:193-205;
  *   use_approx_beliefs LBP.py:554-563 -> au.sparse_dot / sparse_pointwise_multiply / sparse_normalize pyx:108-129, :23-26):
  *   keep the K largest entries of each of the n_rows operand rows A[row0 ..], zero the others (K = 100 in the reference);

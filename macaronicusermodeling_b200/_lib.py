@@ -23,6 +23,7 @@ _SIGNATURES = {
     'mlbp_spike_correct': 'ppppp' + 'ii' + 'ppii' + 'plif' + 'ppf' + 'p',
     'mlbp_topk_mask_rows': 'ppiiliip',
     'mlbp_topk_rows': 'piiiipppp',
+    'mlbp_format_log_rows': 'piiiplpp',
     'mlbp_factor_to_var_gemm': 'pplii' + 'ppii' + 'plifip',
     'mlbp_factor_to_var_gemm_gated': 'pplii' + 'ppii' + 'plifi' + 'pi' + 'ii' + 'f' + 'p',
     'mlbp_marginals': 'ipppp' + 'ppii' + 'ppppf' + 'iff' + 'ppppp' + 'p',

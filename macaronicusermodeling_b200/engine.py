@@ -39,6 +39,7 @@ D_CONST_ROWS = 5
 # one marginals launch, and the re-score counters (mlbp_rescore_candidates)
 FLAG_PEAK, FLAG_NFLAGGED, FLAG_MAXBITS, FLAG_SPIKE, FLAG_NSPIKY, FLAG_COUNTERS, FLAG_WORDS = 0, 1, 2, 3, 4, 8, 16
 SPIKE_SLOTS = 4               # include/mlbp.h MLBP_SPIKE_SLOTS
+FMT_MAX_BYTES = 12            # include/mlbp.h MLBP_FMT_MAX_BYTES: text bytes per number that mlbp_format_log_rows may need
 
 
 def round_up(x, m):
@@ -880,6 +881,19 @@ class Engine(object):
                     lambda: self.k.call('mlbp_topk_rows', _p(X), int(X.stride(0)), self.V, n, int(K), _p(idx), _p(val), _p(ties)))
         self.launches += 1
         return idx, val, ties
+
+    def format_log_rows(self, X):
+        """The .dist numbers of every row of the fp32 device matrix X[:, :V] as text, made on the device (mlbp_format_log_rows;
+        FactorGraph.to_dist, LBP.py:125-143): (text uint8, offsets int64 [n + 1]) device tensors, row r is
+        text[offsets[r]:offsets[r + 1]] = ' '.join('%0.6f' % x for x in np.log(row.astype(np.float64)))."""
+        n = int(X.shape[0])
+        text = torch.empty(max(FMT_MAX_BYTES * self.V * n, 1), dtype=torch.uint8, device=self.device)
+        offsets = torch.empty(n + 1, dtype=torch.int64, device=self.device)
+        self._timed('K7 format_log_rows', n * self.V * 4.0,
+                    lambda: self.k.call('mlbp_format_log_rows', _p(X), int(X.stride(0)), self.V, n, _p(text), int(text.numel()),
+                                        _p(offsets)))
+        self.launches += 1
+        return text, offsets
 
     # ------------------------------------------------------------------ micro-batching
     def microbatches(self, corpus, sweeps, want_grad):

@@ -10,7 +10,8 @@ read (LBP.py:109-143).
 Where train_mp.py hands sentences to `--cpu N` pool workers that each see a theta about N sentences old
 (train_mp.py:634-649), this trainer takes synchronous minibatches of `--minibatch` sentences (default: the value of
 --cpu, 4) that all see the same theta; `--minibatch 1` is train.py's exact per-sentence SGD.  Under torchrun the
-minibatch is sharded over the ranks and the gradient all-reduced (trainer.Trainer).
+minibatch is sharded over the ranks and the gradient all-reduced (trainer.Trainer); prediction (and the --tune pass)
+shares its 64-sentence chunks out over the ranks and writes the files one process writes (predict).
 """
 import argparse
 import codecs
@@ -140,51 +141,165 @@ def draw_roots(corpus, sweeps, rng):
     return np.array([[rng.randrange(int(kk)) for _ in range(1 + sweeps)] for kk in k], dtype=np.int32)
 
 
-def predict(engine, sents, raw, en_domain, de_domain, options, rng, qp, batch=64):
-    """train.py:308-338 batched: returns (sum log-posterior, prediction strings, dist strings, (p0, p25, p50, total))"""
+def prediction_units(n_sents, doms=None, batch=64):
+    """The engine calls of a prediction pass in the order one process makes them: (domain, sentence indices) per chunk of
+    `batch` sentences -- of the whole file, or (--user_adapt / --experience_adapt) of each domain's sentences, domains sorted.
+    Under torchrun the ranks share out these units, so every chunk is the same engine call whatever the number of ranks."""
+    if doms is None:
+        return [(None, list(range(lo, min(lo + batch, n_sents)))) for lo in range(0, n_sents, batch)]
+    units = []
+    for d in sorted(set(doms)):
+        idx = [i for i, x in enumerate(doms) if x == d]
+        units += [(d, idx[lo:lo + batch]) for lo in range(0, len(idx), batch)]
+    return units
+
+
+def dist_text(engine, beliefs, pinned):
+    """The .dist numbers of a chunk's belief rows, formatted on the device (mlbp_format_log_rows) and copied back at once into
+    the pinned buffer pinned[0] (grown as needed): (uint8 array, int64 row offsets [n + 1]) on the host."""
+    import torch
+    text, off = engine.format_log_rows(beliefs)
+    off = off.cpu().numpy()
+    total = int(off[-1])
+    if pinned[0] is None or pinned[0].numel() < total:
+        pinned[0] = None
+        pinned[0] = torch.empty(total + total // 4 + 1, dtype=torch.uint8, pin_memory=engine.device.type == 'cuda')
+    host = pinned[0][:total]
+    host.copy_(text[:total])
+    return host.numpy(), off
+
+
+def merge_parts(path, parts, spans):
+    """The final file from the ranks' part files: spans[i] = (rank, offset, length) of sentence i, in file order.  The part
+    files are removed."""
+    import os
+    runs = []
+    for rk, off, ln in spans:
+        if runs and runs[-1][0] == rk and runs[-1][1] + runs[-1][2] == off:
+            runs[-1][2] += ln
+        else:
+            runs.append([rk, off, ln])
+    if len(runs) == 1 and runs[0][1] == 0 and runs[0][2] == os.path.getsize(parts[runs[0][0]]):
+        os.replace(parts[runs[0][0]], path)                    # one part holds the whole file in order: no copy
+    else:
+        srcs = [open(p, 'rb') for p in parts]
+        try:
+            with open(path, 'wb') as w:
+                for rk, off, ln in runs:
+                    srcs[rk].seek(off)
+                    while ln > 0:
+                        b = srcs[rk].read(min(ln, 1 << 24))
+                        if not b:
+                            raise IOError('%s is shorter than the spans written to it' % parts[rk])
+                        w.write(b)
+                        ln -= len(b)
+        finally:
+            for f in srcs:
+                f.close()
+    for p in parts:
+        if os.path.exists(p):
+            os.remove(p)
+
+
+def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None, out_path=None):
+    """train.py:308-338 batched and sharded over the torchrun ranks.  `units`: prediction_units(); `thetas`: domain ->
+    (theta_ee, theta_ed) for the adaptation modes (else the engine's current theta is used).  The roots of every sentence are
+    drawn from `rng` in unit order before the units are shared out, so a sentence gets the same roots on any number of ranks.
+    Rank r runs units r, r + world, ...; with `out_path` (and not qp) each rank writes its sentences' .pred / .dist text
+    to part files next to the output, and after a barrier rank 0 merges them in file order.  Returns the all-reduced
+    (sum log-posterior, (p0, p25, p50, total)) on every rank, summed in the order one process sums them."""
+    import torch
     from .engine import Corpus
-    logp_sum, preds, dists = 0.0, [], []
-    p0 = p25 = p50 = tot = 0
+    from .trainer import dist_info
+    rank, world = dist_info()
     V = len(en_domain)
-    for lo in range(0, len(sents), batch):
-        chunk = sents[lo:lo + batch]
-        corpus = Corpus(chunk)
-        r = engine.run(corpus, draw_roots(corpus, 3, rng), 3, want_grad=False, want_marg=True, want_beliefs=not qp,
+    corpora = [Corpus([sents[i] for i in idx]) for _, idx in units]
+    roots = [draw_roots(c, 3, rng) for c in corpora]
+    stats = np.zeros((len(units), 5))                           # per unit: sum logp, #rank == 0, < 26, < 50, variables
+    write = bool(out_path) and not qp
+    if write:
+        parts = [out_path + '.rank%d.part' % r for r in range(world)]
+        dparts = [out_path + '.dist.rank%d.part' % r for r in range(world)]
+        wp, wd = open(parts[rank], 'wb'), open(dparts[rank], 'wb')
+        spans, p_off, d_off = [], 0, 0                          # (sentence, .pred offset, length, .dist offset, length)
+    pinned = [None]
+    cur = object()
+    for u in range(rank, len(units), world):
+        dom, idx = units[u]
+        if thetas is not None and dom != cur:
+            engine.set_theta(thetas[dom][0], thetas[dom][1], with_grad=True)
+            cur = dom
+        corpus = corpora[u]
+        r = engine.run(corpus, roots[u], 3, want_grad=False, want_marg=True, want_beliefs=not qp,
                        approx_inference=options.use_approx_inference, want_topk=0 if qp else min(50, V - 1))
-        logp_sum += float(r.logp.sum().item())
-        rank = r.rank.cpu().numpy()
-        p0 += int((rank == 0).sum()); p25 += int((rank < 26).sum()); p50 += int((rank < 50).sum()); tot += len(rank)
-        if qp:
+        rk = r.rank.cpu().numpy()
+        stats[u] = (float(r.logp.sum().item()), int((rk == 0).sum()), int((rk < 26).sum()), int((rk < 50).sum()), len(rk))
+        if not write:
             continue
+        text, toff = dist_text(engine, r.beliefs, pinned)
         B = r.beliefs.cpu().numpy()[:, :V].astype(np.float64)
         TI, _, TT = (x.cpu().numpy() for x in r.topk)        # the 50 best words per variable, listed on the device (mlbp_topk_rows)
-        for si, s in enumerate(chunk):
-            ti = raw[lo + si]
+        for si, i in enumerate(idx):
+            s, ti = sents[i], raw[i]
             nodes = sorted(ti['current_sent'], key=lambda n: int(n['position']))
-            lines, dl = ['*SENT_ID:' + str(nodes[0]['sent_id'])], []
+            lines = ['*SENT_ID:' + str(nodes[0]['sent_id'])]
             vi = int(corpus.var_off[si])
+            d_len = 0
             for p, n in enumerate(nodes):                                            # FactorGraph.to_string, LBP.py:109-123
                 if s.kind[p] == 1:
                     b = B[vi]
                     vi += 1
                     top = min(50, V - 1)
                     if TT[vi - 1] == 0:
-                        idx = TI[vi - 1]
+                        idx_top = TI[vi - 1]
                     else:                                    # exact ties: the reference's order is NumPy's (LBP.py:405-406)
-                        idx = np.argpartition(b, -top)[-top:]
-                        idx = idx[np.argsort(b[idx])][::-1]
+                        idx_top = np.argpartition(b, -top)[-top:]
+                        idx_top = idx_top[np.argsort(b[idx_top])][::-1]
                     with np.errstate(divide='ignore'):
                         lb = np.log(b)
                     sl = en_domain[int(s.label[p])]
-                    pred = ' '.join(en_domain[i] + ' ' + '%0.4f' % lb[i] for i in idx)
+                    pred = ' '.join(en_domain[e] + ' ' + '%0.4f' % lb[e] for e in idx_top)
                     lines.append(' '.join([n['l2_word'], sl, '%0.4f' % lb[int(s.label[p])], pred]))
                     truth = n['l1_parent'].lower().replace("'", "") if n.get('l1_parent') else 'None'
-                    dl.append(' ||| '.join([truth, sl, ' '.join('%0.6f' % x for x in lb)]))   # to_dist, LBP.py:125-143
+                    # to_dist, LBP.py:125-143: "truth ||| label ||| " + the numbers made on the device
+                    head = ('\n' if d_len else '') + ' ||| '.join([truth, sl, ''])
+                    d_len += wd.write(head.encode('utf8')) + wd.write(text[toff[vi - 1]:toff[vi]])
                 else:
                     lines.append(' '.join(['', en_domain[int(s.label[p])], '']))
-            preds.append('\n'.join(lines))
-            dists.append('\n'.join(dl))
-    return logp_sum, preds, dists, (p0, p25, p50, tot)
+            d_len += wd.write(b'\n')
+            p_len = wp.write(('\n'.join(lines) + '\n').encode('utf8'))
+            spans.append((i, p_off, p_len, d_off, d_len))
+            p_off += p_len
+            d_off += d_len
+    if world > 1:
+        import torch.distributed as dist
+        red = torch.from_numpy(stats).to(engine.device)        # every unit is non-zero on exactly one rank: the sums are exact
+        dist.all_reduce(red, op=dist.ReduceOp.SUM)
+        stats = red.cpu().numpy()
+    if write:
+        wp.close()
+        wd.close()
+        every = [spans]
+        if world > 1:
+            every = [None] * world
+            dist.all_gather_object(every, spans)
+            dist.barrier()                                      # every part file is closed
+        if rank == 0:
+            where = [None] * len(sents)
+            for rr, sp in enumerate(every):
+                for i, po, pl, do, dl in sp:
+                    where[i] = (rr, po, pl, do, dl)
+            merge_parts(out_path, parts, [(w[0], w[1], w[2]) for w in where])
+            merge_parts(out_path + '.dist', dparts, [(w[0], w[3], w[4]) for w in where])
+    logp_sum, k = 0.0, 0
+    while k < len(units):                                       # one partial sum per domain, as the single-process loop
+        part, d = 0.0, units[k][0]
+        while k < len(units) and units[k][0] == d:
+            part += float(stats[k, 0])
+            k += 1
+        logp_sum += part
+    c = stats[:, 1:].sum(axis=0) if len(units) else np.zeros(4)
+    return logp_sum, tuple(int(x) for x in c)
 
 
 def main(argv=None):
@@ -205,7 +320,8 @@ def main(argv=None):
     # one process per GPU under torchrun: rank / world from the environment, NCCL over NVLink for the 16 x f64 all-reduce
     if int(os.environ.get('WORLD_SIZE', '1')) > 1:
         import torch.distributed as dist
-        torch.cuda.set_device(int(os.environ.get('LOCAL_RANK', '0')))
+        if torch.cuda.is_available():
+            torch.cuda.set_device(int(os.environ.get('LOCAL_RANK', '0')))
         if not dist.is_initialized():
             os.environ.setdefault('MASTER_ADDR', '127.0.0.1')
             dist.init_process_group('nccl' if torch.cuda.is_available() else 'gloo')
@@ -303,11 +419,13 @@ def main(argv=None):
                 print('saved params')
             if tune_lines is not None:
                 engine.set_theta(tr.theta_ee, tr.theta_ed, with_grad=True)
-                lp, _, _, (p0, p25, p50, tot) = predict(engine, lower(tune_lines, options, en2id, de2id),
-                                                        [json.loads(l) for l in tune_lines], en_domain, de_domain, options, rng, True)
-                print('\ntune prediction probs:', lp / float(len(tune_lines)))
-                for name, p in (('Prec at 0:', p0), ('prec at 25:', p25), ('prec at 50:', p50)):
-                    print(name, '%0.2f' % (float(100 * p) / float(max(tot, 1))), 'total:', tot)
+                tune_sents = lower(tune_lines, options, en2id, de2id)
+                lp, (p0, p25, p50, tot) = predict(engine, prediction_units(len(tune_sents)), tune_sents,
+                                                  [json.loads(l) for l in tune_lines], en_domain, options, rng, True)
+                if rank == 0:
+                    print('\ntune prediction probs:', lp / float(len(tune_lines)))
+                    for name, p in (('Prec at 0:', p0), ('prec at 25:', p25), ('prec at 50:', p50)):
+                        print(name, '%0.2f' % (float(100 * p) / float(max(tot, 1))), 'total:', tot)
         print('\ntheta final:', tr.theta_ee, tr.theta_ed)
         if rank == 0 and options.save_params_file:
             save_params(codecs.open(options.save_params_file, 'w', 'utf8'), tr.theta_ee.reshape(1, -1), tr.theta_ed.reshape(1, -1),
@@ -319,31 +437,19 @@ def main(argv=None):
     if adapt:
         # every sentence is scored with its domain's theta (train.py:224-245 via create_factor_graph); results keep file order
         doms = [domain_of(r, options) for r in raw]
-        lp, p0, p25, p50, tot = 0.0, 0, 0, 0, 0
-        preds, dists = [None] * len(raw), [None] * len(raw)
-        for d in sorted(set(doms)):
-            idx = [i for i, x in enumerate(doms) if x == d]
-            engine.set_theta(d2t_loaded['en_en', d].reshape(-1), d2t_loaded['en_de', d].reshape(-1), with_grad=True)
-            l_, pr, di, (a0, a25, a50, at) = predict(engine, [all_sents[i] for i in idx], [raw[i] for i in idx], en_domain,
-                                                     de_domain, options, rng, options.quick_predict)
-            lp += l_; p0 += a0; p25 += a25; p50 += a50; tot += at
-            for j, i in enumerate(idx):
-                if pr:
-                    preds[i], dists[i] = pr[j], di[j]
+        thetas = dict((d, (d2t_loaded['en_en', d].reshape(-1), d2t_loaded['en_de', d].reshape(-1))) for d in set(doms))
+        units = prediction_units(len(all_sents), doms)
     else:
         engine.set_theta(theta_ee.reshape(-1), theta_ed.reshape(-1), with_grad=True)
-        lp, preds, dists, (p0, p25, p50, tot) = predict(engine, all_sents, raw, en_domain, de_domain, options, rng,
-                                                         options.quick_predict)
-    if not options.quick_predict:
-        with codecs.open(options.save_predictions_file, 'w', 'utf8') as w, \
-                codecs.open(options.save_predictions_file + '.dist', 'w', 'utf8') as wd:
-            for p, d in zip(preds, dists):
-                w.write(p + '\n')
-                wd.write(d + '\n')
-    print('\nprediction probs:', lp / float(len(train_lines)))
-    for name, p in (('Prec at 0:', p0), ('prec at 25:', p25), ('prec at 50:', p50)):
-        print(name, '%0.2f' % (float(100 * p) / float(max(tot, 1))), 'total:', tot)
-    torch.cuda.synchronize()
+        thetas, units = None, prediction_units(len(all_sents))
+    lp, (p0, p25, p50, tot) = predict(engine, units, all_sents, raw, en_domain, options, rng, options.quick_predict, thetas,
+                                      options.save_predictions_file)
+    if rank == 0:
+        print('\nprediction probs:', lp / float(len(train_lines)))
+        for name, p in (('Prec at 0:', p0), ('prec at 25:', p25), ('prec at 50:', p50)):
+            print(name, '%0.2f' % (float(100 * p) / float(max(tot, 1))), 'total:', tot)
+    if torch.cuda.is_available():
+        torch.cuda.synchronize()
     return 0
 
 

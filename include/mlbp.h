@@ -182,6 +182,36 @@ int mlbp_topk_rows(const float *X, int ldx, int V, int n_rows, int K, int32_t *i
 #define MLBP_FMT_MAX_BYTES   12   /* "-103.278930" (log of the smallest subnormal) plus its separator                 */
 int mlbp_format_log_rows(const float *X, int ldx, int V, int n_rows, char *out, int64_t out_bytes, int64_t *offsets,
                          void *stream);
+/* K8.  np.loadtxt(path, dtype=float64) of a feature matrix (train.py:589-603) on the device, one chunk of the file at a time:
+ *   text[0 .. n_bytes) (16-byte aligned) starts at byte file_offset of the file and ends on a line boundary (after a '\n', or
+ *   at the end of the file).  Grammar, for ASCII text: fields separated by runs of ' ' \t \v \f (and \r before \n); blank and
+ *   whitespace-only lines are skipped; '#' starts a comment that runs to the end of the line; a field is
+ *   [+-] (digits [. digits] | . digits) [(e|E) [+-] digits] or [+-] (inf | infinity | nan), case-insensitive.
+ *   Field k of the file (state[MLBP_PARSE_FIELDS] counts the fields of the earlier chunks) is converted to the correctly rounded
+ *   float64, rounded to nearest-even fp32 and stored at out[row * ld_out + col], (row, col) = divmod(k, n_cols); NaN keeps its sign.
+ *   state: MLBP_PARSE_STATE_WORDS device words, zeroed by the caller before the first chunk of a file and read once after the
+ *   last:  [MLBP_PARSE_FIELDS] fields so far; [MLBP_PARSE_ERROR] ~(offset << 3 | kind) of the first offending byte (0 = none);
+ *   [MLBP_PARSE_MIN] ~key of the smallest value, [MLBP_PARSE_MAX] key of the largest (key(b) = b ^ (sign ? ~0 : 1 << 63) of the
+ *   float64 bits b; NaN and hard fields are not included); [MLBP_PARSE_NAN] bit 0 / 1: a positive / negative NaN was read;
+ *   [MLBP_PARSE_HARD] number of hard fields.
+ *   Hard fields (more than 19 significant digits whose rounding the first 19 do not decide) are not written: their (file byte
+ *   offset, field index) pairs go to hard[2 * i], hard[2 * i + 1] for i < hard_cap, in no particular order; the caller converts them.
+ *   tile_ws: ceil(n_bytes / MLBP_PARSE_TILE_BYTES) device words of scratch.  n_bytes <= MLBP_PARSE_MAX_CHUNK.             */
+#define MLBP_PARSE_TILE_BYTES   4096
+#define MLBP_PARSE_MAX_CHUNK    (((int64_t)1 << 31) - 1)
+#define MLBP_PARSE_STATE_WORDS  8
+#define MLBP_PARSE_FIELDS       0
+#define MLBP_PARSE_ERROR        1
+#define MLBP_PARSE_MIN          2
+#define MLBP_PARSE_MAX          3
+#define MLBP_PARSE_NAN          4
+#define MLBP_PARSE_HARD         5
+#define MLBP_PARSE_ERR_FIELD    1   /* a field outside the grammar                                  */
+#define MLBP_PARSE_ERR_COLS     2   /* a line whose field count is not n_cols                        */
+#define MLBP_PARSE_ERR_ROWS     3   /* more than max_rows rows                                       */
+#define MLBP_PARSE_ERR_BYTE     4   /* a byte >= 0x80, another control byte, or \r not before \n      */
+int mlbp_parse_float_text(const char *text, int64_t n_bytes, int64_t file_offset, int n_cols, int64_t max_rows, float *out,
+                          int64_t ld_out, uint64_t *state, int64_t *hard, int hard_cap, uint64_t *tile_ws, void *stream);
 /* Approximate paths (use_approx_inference LBP.py:506-507, :515-516 -> au.sparse_vec_mat_dot pyx:193-205;
  *   use_approx_beliefs LBP.py:554-563 -> au.sparse_dot / sparse_pointwise_multiply / sparse_normalize pyx:108-129, :23-26):
  *   keep the K largest entries of each of the n_rows operand rows A[row0 ..], zero the others (K = 100 in the reference);

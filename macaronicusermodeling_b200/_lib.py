@@ -24,6 +24,7 @@ _SIGNATURES = {
     'mlbp_topk_mask_rows': 'ppiiliip',
     'mlbp_topk_rows': 'piiiipppp',
     'mlbp_format_log_rows': 'piiiplpp',
+    'mlbp_parse_float_text': 'plli' + 'lpl' + 'ppip' + 'p',
     'mlbp_factor_to_var_gemm': 'pplii' + 'ppii' + 'plifip',
     'mlbp_factor_to_var_gemm_gated': 'pplii' + 'ppii' + 'plifi' + 'pi' + 'ii' + 'f' + 'p',
     'mlbp_marginals': 'ipppp' + 'ppii' + 'ppppf' + 'iff' + 'ppppp' + 'p',

@@ -12,6 +12,7 @@ Data layout in HBM (all rows padded to ld = roundup(V, 64) elements):
     D       [RD, ld] fp32   factor->variable messages, one row per GEMM row (K4 -> K3/K5/K6)
 PyTorch is used for device memory and streams only; all arithmetic is in libmlbp.so.
 """
+import contextlib
 import ctypes
 import math
 import os
@@ -95,6 +96,22 @@ class Model(object):
     @classmethod
     def from_dict(cls, m, device):
         return cls(m['pmi'], m['pmi_w1'], m['ed'], m['ped'], device)
+
+    @classmethod
+    def from_text(cls, pmi, pmi_w1, ed, ped, V, Vd, device=None, chunk_bytes=None, kernels=None):
+        """The model that Model(*[np.loadtxt(p, dtype=np.float64, ndmin=2) for p in (pmi, pmi_w1, ed, ped)], device) builds,
+        with the text parsed on the GPU (textload.py, K8): pmi / pmi_w1 [V, V] and ed / ped [V, Vd] text files.  A file
+        that is not a clean V-row matrix in the device grammar is read with np.loadtxt instead (one RuntimeWarning).
+        chunk_bytes: size of the two pinned read buffers (default 256 MB).  A back end whose device is not a GPU (the
+        emulated kernels of the CPU test tier) has nothing to parse on: it gets the np.loadtxt path."""
+        from . import textload
+        paths = (pmi, pmi_w1, ed, ped)
+        cuda = device is not None and torch.device(device).type == 'cuda'
+        with torch.cuda.device(torch.device(device)) if cuda else contextlib.nullcontext():
+            k = kernels or Kernels()
+            if k.device.type != 'cuda':
+                return cls(*[np.loadtxt(p, dtype=np.float64, ndmin=2) for p in paths], device=k.device)
+            return textload.model_from_text(cls, paths, V, Vd, k, chunk_bytes)
 
 
 class Corpus(object):

@@ -76,15 +76,13 @@ def error_msg():
 
 
 def load_inputs(options):
+    from .engine import Model
     de_domain = [i.strip() for i in codecs.open(options.de_domain, 'r', 'utf8').readlines()]       # train.py:582-585
     en_domain = [i.strip() for i in codecs.open(options.en_domain, 'r', 'utf8').readlines()]
     en2id = dict((e, idx) for idx, e in enumerate(en_domain))
     de2id = dict((d, idx) for idx, d in enumerate(de_domain))
-    model = {'pmi': np.loadtxt(options.phi_pmi, dtype=np.float64, ndmin=2),                        # train.py:589-603
-             'pmi_w1': np.loadtxt(options.phi_pmi_w1, dtype=np.float64, ndmin=2),
-             'ed': np.loadtxt(options.phi_ed, dtype=np.float64, ndmin=2),
-             'ped': np.loadtxt(options.phi_ped, dtype=np.float64, ndmin=2)}
-    model['V'], model['Vd'] = len(en_domain), len(de_domain)
+    # train.py:589-603 np.loadtxt's the four matrices; they are parsed on the device into the same planes (textload.py)
+    model = Model.from_text(options.phi_pmi, options.phi_pmi_w1, options.phi_ed, options.phi_ped, len(en_domain), len(de_domain))
     return en_domain, de_domain, en2id, de2id, model
 
 

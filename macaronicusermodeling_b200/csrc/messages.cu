@@ -77,7 +77,9 @@ var_to_factor_kernel(const int32_t *__restrict__ grp_u, const int32_t *__restric
     __shared__ int s_d0[NMAX], s_nd[NMAX];
     __shared__ size_t s_first[NMAX];
     __shared__ double s_warp[K3_WARPS][NMAX];
-    __shared__ float s_scale[NMAX];
+    // the normaliser in T: in fp64 the sums reach far outside the fp32 range (2^14 / t is 0 above t = 2^163, inf below
+    // t = 2^-114), and a float scale would turn those messages uniform or infinite
+    __shared__ T s_scale[NMAX];
     const int g = blockIdx.x;
     const int i0 = grp_off[g], n = grp_off[g + 1] - i0;
     const float *urow = U + (size_t)grp_u[g] * ldv;
@@ -125,7 +127,7 @@ var_to_factor_kernel(const int32_t *__restrict__ grp_u, const int32_t *__restric
 #pragma unroll
         for (int w = 0; w < K3_WARPS; ++w) t += s_warp[w][threadIdx.x];
         // sum <= 0 or non-finite -> uniform (Message.renormalize, LBP.py:650-657); flagged by a negative scale
-        s_scale[threadIdx.x] = (t > 0.0 && isfinite(t)) ? (float)(ldexp(1.0, MLBP_A_SCALE_LOG2) / t) : -1.0f;
+        s_scale[threadIdx.x] = (t > 0.0 && isfinite(t)) ? (T)(ldexp(1.0, MLBP_A_SCALE_LOG2) / t) : (T)-1;
     }
     __syncthreads();
 
@@ -145,8 +147,8 @@ var_to_factor_kernel(const int32_t *__restrict__ grp_u, const int32_t *__restric
         for (int j = NMAX - 1; j >= 0; --j) {
             const int nd = s_nd[j];                               // 0 beyond n and for messages nobody reads
             if (nd > 0) {
-                const float sc = s_scale[j];
-                const float x = sc > 0.f ? (float)(pre[j] * suf * (T)sc) : uni;
+                const T sc = s_scale[j];
+                const float x = sc > (T)0 ? (float)(pre[j] * suf * sc) : uni;
                 k3_store(x, s_first[j] + e, nd, dest, s_d0[j], ldv, e, A_hi, A_lo);
             }
             suf *= (T)d[j];

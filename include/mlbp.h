@@ -314,6 +314,25 @@ int mlbp_gradient_reduce(int n_sent, const int32_t *sent_var_off, const int32_t 
  *   One CTA, fixed summation order (deterministic).                                                              */
 int mlbp_batch_reduce(int n_sent, const double *grad, const double *logp_sent, int n_vars, const int32_t *rank,
                       const int32_t *peak_flag, double *out16, void *stream);
+/* K9.  Joint log-likelihood of each sentence's labels, the Bethe estimate at the final messages (not in the reference, whose
+ *   one fit statistic is the sum of MARGINAL log-probabilities, LBP.py:247-259):
+ *     logp_joint[s] = sum_{v in s} logp_var[v]
+ *                   + sum_{pairwise f in s} [ log T_f(y0, y1) - log Z_f + sum_{k = 0, 1} ( log O_{f,k} - log mu_k[y_k] ) ]
+ *   with y0, y1 = var_label[pair_v0[f]], var_label[pair_v1[f]]; nu_0 = (A_hi + A_lo)[c_row[f]], nu_1 = (A_hi + A_lo)[r_row[f]]
+ *   the final variable->factor messages, mu_k = D[mk_row[f]] (mk_row < 0: the constant-one row D[0]) the final factor->variable
+ *   messages of the factor's dim-0 / dim-1 variable, O_{f,k} = nu_k . mu_k (fp32 products, float64 sums in a fixed order),
+ *   Z_f = pair_stats[f][0] * 2^-z_scale_log2 (mlbp_pair_expectations: 2^z_scale_log2 * nu_0' T nu_1 on the unscaled table),
+ *   log T = th[0] * pmi + th[1] * pmi_w1 (gap == 1 only) + th[2] in float64 from the fp32 planes [V, ldf] (train.py:218-219).
+ *   Row scales cancel (each row enters once with + and once with -).  Exact on trees; with one variable it is logp_var.
+ *   A sentence with a variable whose logp_var is -99.99 (label of belief 0) gets -inf.  pair_term: n_pairs float64 of scratch.
+ *   Sentence s owns variables [sent_var_off[s], ..) and factors [sent_fac_off[s], ..); n_pairs = sent_fac_off[n_sent].
+ *   Two launches (one warp per factor, one warp per sentence), deterministic.  Bad arguments: MLBP_ERR_INVALID, nothing launched. */
+int mlbp_joint_logp(int n_sent, int n_pairs, const int32_t *sent_var_off, const int32_t *sent_fac_off, const double *logp_var,
+                    const int32_t *c_row, const int32_t *r_row, const int32_t *m0_row, const int32_t *m1_row,
+                    const int32_t *pair_v0, const int32_t *pair_v1, const int32_t *var_label, const int32_t *pair_gap1,
+                    const double *pair_stats, const void *A_hi, const void *A_lo, const float *D, int ldv, int V,
+                    const float *pmi, const float *pmi_w1, int ldf, const double *h_theta_ee, int z_scale_log2,
+                    double *pair_term, double *logp_joint, void *stream);
 /* rows[0] = 1.0f (the constant-one row the kernels read for a message that is still uniform), rows[1 + t] = the message of a
  *   pairwise factor of message table t (MLBP_TABLE_T .. T1T) that is fed the uniform initial message (LBP.py:211-216 +
  *   :509 / :518): the row / column sums of the table, mean-one scaled.  rows: [MLBP_D_CONST_ROWS, ldv] fp32; the engine
@@ -344,7 +363,9 @@ typedef struct mlbp_plan mlbp_plan;
  * flags: bit 0 = plan the gradient stage, bit 1 = plan the marginal stage, bit 2 = do NOT constant-fold updates
  *        that read an initial uniform message (needed by the top-K approximate mode, which masks that message),
  *        bit 3 = give every pairwise belief normaliser Z its own GEMM row instead of reusing the D row of the factor's
- *        last message update (needed whenever message rows are masked: top-K approximate modes).              */
+ *        last message update (needed whenever message rows are masked: top-K approximate modes),
+ *        bit 4 = with bits 0 and 1: also emit, per pairwise factor, the D rows of its final factor->variable messages (blob
+ *        header words 29 / 30; what mlbp_joint_logp reads as m0_row / m1_row).  Without it the blob is unchanged.       */
 int mlbp_plan_compile(int n_graphs, const int32_t *h_var_off, const int32_t *h_pair_off, const int32_t *h_pair_v0,
                       const int32_t *h_pair_v1, const int32_t *h_pair_gap1, const int32_t *h_roots, int sweeps,
                       int flags, mlbp_plan **out);

@@ -118,6 +118,7 @@ class FactorGraph():
         self._sweeps = 0
         self._initialized = False
         self._res = None          # cached engine outputs for (_sweeps, theta snapshot)
+        self._joint = None        # (key, get_joint_log_likelihood())
         self._messages = None
         # Eager mode: the reference's one-message-at-a-time API (VariableNode / FactorNode.update_message_to) and
         # graphs with explicit PotentialTable(table=...) arrays.  graph.messages then IS the state, every update is
@@ -144,7 +145,7 @@ class FactorGraph():
             if v.id not in self.variables:
                 self.variables[v.id] = v
                 v.graph = self
-        self._res = None
+        self._res = self._joint = None
 
     def get_message_schedule(self, root):
         """The (child, parent) edge list one sweep walks (reference: LBP.py:155-172).  Breadth-first from `root` with the
@@ -213,7 +214,7 @@ class FactorGraph():
         self._roots = [self._last_loop_root]
         self._sweeps = 0
         self._initialized = True
-        self._res = None
+        self._res = self._joint = None
         self._messages = None
         self._eager = self._uniform_messages() if self._explicit else None
 
@@ -237,7 +238,7 @@ class FactorGraph():
             if not self._initialized:
                 raise KeyError('messages are not initialised: call initialize() first')
             self._eager = self._uniform_messages() if self._sweeps == 0 else dict(self.messages)
-            self._res = None
+            self._res = self._joint = None
             self._messages = None
         return self._eager
 
@@ -260,7 +261,7 @@ class FactorGraph():
                     if not (isinstance(to, FactorNode) and len(to.varset) < 2):
                         frm.update_message_to(to)
             if self.report_times: self.it_times.append(time.time() - it)
-        self._res = None
+        self._res = self._joint = None
         self._messages = None
         return True
 
@@ -424,6 +425,28 @@ class FactorGraph():
                 sys.stderr.write('err -inf' + str(0.0))
             log_posterior += float(_l)
         return log_posterior
+
+    def get_joint_log_likelihood(self):
+        """Not in the reference: the joint log-likelihood of the supervised labels, log p(y) with
+        p(y) ~ prod U_i(y_i) prod T_F(y_i, y_j), as loopy BP estimates it (Bethe free energy at the final messages; exact on
+        trees).  get_posterior_probs is the sum of per-variable MARGINAL log-probabilities instead.  -inf when a label has
+        belief 0.  Lazy batched mode only; the approximate modes are refused (ValueError)."""
+        if self._eager is not None or self._explicit:
+            raise NotImplementedError('the joint log-likelihood is computed on the device from the batched run: not available '
+                                      'with explicit potential tables or once messages were set or updated by hand')
+        if self.use_approx_inference or self.use_approx_beliefs:
+            raise ValueError('the joint log-likelihood is not defined for the approximate modes')
+        key = (self._sweeps, self._theta_key(), tuple(self._roots))
+        if self._joint is None or self._joint[0] != key:
+            if not self._initialized:
+                raise KeyError('messages are not initialised: call initialize() first')
+            eng = _engine_for(self)
+            corpus, _, _ = self._lower()
+            eng.set_theta(*self._pot_thetas())
+            r = eng.run(corpus, corpus.roots_from_positions([list(self._roots)]), self._sweeps, want_grad=False,
+                        want_marg=True, want_joint=True)
+            self._joint = (key, float(r.logp_joint[0].item()))
+        return self._joint[1]
 
     def get_max_postior_label(self, top=10):
         label_guesses = []

@@ -34,6 +34,7 @@ _SIGNATURES = {
     'mlbp_gradient_reduce': 'ippppppp' + 'p' + 'ppi' + 'pppp',
     'mlbp_batch_reduce': 'ippipppp',
     'mlbp_const_rows': 'piipp',
+    'mlbp_joint_logp': 'ii' + 'ppp' + 'pppp' + 'pppp' + 'ppppii' + 'ppi' + 'pi' + 'pp' + 'p',
     'mlbp_plan_compile': 'ipppppp' + 'iip',
     'mlbp_plan_sizes': 'pp',
     'mlbp_plan_export': 'pp',

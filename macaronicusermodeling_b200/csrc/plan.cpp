@@ -51,7 +51,8 @@ namespace {
 enum {
     H_NLEVELS = 0, H_LEVELS_OFF, H_INIT_N, H_INIT_OFF, H_NPAIR, H_PAIR_C, H_PAIR_U0, H_PAIR_U1, H_PAIR_U2, H_PAIR_GAP1,
     H_PAIR_V0, H_PAIR_V1, H_NGRAD_GEMM, H_GRAD_GEMM_OFF, H_MARG_N, H_MARG_U, H_MARG_OFF, H_MARG_IN, H_NGRAPHS,
-    H_A_ROWS, H_D_ROWS, H_MAX_IN, H_NVARS, H_PAIR_R, H_PAIR_Z, H_MSG_BLK_N, H_MSG_BLK_OFF, H_MSG_ROWS, H_SPK_BLK_N, H_WORDS = 32
+    H_A_ROWS, H_D_ROWS, H_MAX_IN, H_NVARS, H_PAIR_R, H_PAIR_Z, H_MSG_BLK_N, H_MSG_BLK_OFF, H_MSG_ROWS, H_SPK_BLK_N, H_PAIR_M0,
+    H_PAIR_M1, H_WORDS = 32
 };
 enum { LEV_NGROUPS = 0, LEV_GRP_U, LEV_GRP_OFF, LEV_IN_ROW, LEV_DEST_OFF, LEV_DEST, LEV_NGEMM, LEV_GEMM, LEV_FIRST, LEV_SECOND, LEV_WORDS = 10 };
 enum { GEMM_TABLE = 0, GEMM_A0, GEMM_D0, GEMM_N, GEMM_WORDS = 4 };
@@ -218,6 +219,7 @@ void build_sequence(Graph &g, const int32_t *roots, int sweeps) {
 struct ChunkOut {
     std::vector<std::vector<int32_t>> grp_u, grp_off, in_row, dest_off, dest, first, second;   // [level]
     std::vector<int32_t> init_rows, pair_c, pair_r, pair_z, pair_u0, pair_u1, pair_u2, pair_g1, pair_gv0, pair_gv1, mu, moff, min_;
+    std::vector<int32_t> pair_m0, pair_m1;                      // flag bit 4: D rows of the final factor->variable messages
     void set_levels(int n_levels) {
         grp_u.resize(n_levels + 1); grp_off.resize(n_levels + 1); in_row.resize(n_levels + 1); dest_off.resize(n_levels + 1);
         dest.resize(n_levels + 1); first.resize(n_levels + 1); second.resize(n_levels + 1);
@@ -240,7 +242,8 @@ struct EmitScratch {
 };
 
 // phase C for ONE graph: global rows, destinations, leave-one-out groups, gradient / marginal index lists appended to `co`
-static void emit_graph(const Graph &g, const Bases &B, bool want_grad, bool want_marg, ChunkOut &co, EmitScratch &sc) {
+static void emit_graph(const Graph &g, const Bases &B, bool want_grad, bool want_marg, bool want_joint, ChunkOut &co,
+                       EmitScratch &sc) {
     auto &dcount = sc.dcount; auto &dstart = sc.dstart; auto &dflat = sc.dflat; auto &ver = sc.ver; auto &tgt = sc.tgt;
     auto &lev_ops = sc.lev_ops;
     if ((int)lev_ops.size() < g.n_levels + 1) lev_ops.resize(g.n_levels + 1);
@@ -337,6 +340,11 @@ static void emit_graph(const Graph &g, const Bases &B, bool want_grad, bool want
             i = j;
         }
     }
+    if (want_joint)                                              // mu rows of the joint log-likelihood (mlbp_joint_logp)
+        for (int f = 0; f < g.np; ++f) {
+            co.pair_m0.push_back(d_row_of(g.fin_f2v[2 * f + 0]));
+            co.pair_m1.push_back(d_row_of(g.fin_f2v[2 * f + 1]));
+        }
     if (want_marg)
         for (int v = 0; v < g.nv; ++v) {
             co.mu.push_back((int32_t)(B.var + v));
@@ -453,7 +461,7 @@ size_t chunk_bytes(const ChunkOut &co) {
     for (auto *vv : {&co.grp_u, &co.grp_off, &co.in_row, &co.dest_off, &co.dest, &co.first, &co.second})
         for (const auto &v : *vv) n += v.capacity();
     for (auto *v : {&co.init_rows, &co.pair_c, &co.pair_r, &co.pair_z, &co.pair_u0, &co.pair_u1, &co.pair_u2, &co.pair_g1,
-                    &co.pair_gv0, &co.pair_gv1, &co.mu, &co.moff, &co.min_})
+                    &co.pair_gv0, &co.pair_gv1, &co.mu, &co.moff, &co.min_, &co.pair_m0, &co.pair_m1})
         n += v->capacity();
     return n * sizeof(int32_t);
 }
@@ -466,7 +474,7 @@ std::shared_ptr<const Tmpl> build_template(int nv, int np, const int32_t *v0, co
     T->nv = nv; T->np = np;
     T->err = analyse_graph(g, nv, np, v0, v1, gap1, r, sweeps, flags, needed, T->n_dead);
     if (T->err) return T;
-    const bool want_grad = flags & 1, want_marg = flags & 2;
+    const bool want_grad = flags & 1, want_marg = flags & 2, want_joint = want_grad && want_marg && (flags & 16);
     T->n_levels = g.n_levels;
     for (int v = 0; v < g.nv; ++v) T->max_in = std::max(T->max_in, (int)g.facset[v].size());
     const size_t LT = (size_t)(g.n_levels + 1) * 4;
@@ -488,7 +496,7 @@ std::shared_ptr<const Tmpl> build_template(int nv, int np, const int32_t *v0, co
     B.c = S(SEG_C); B.u2z = S(SEG_U2Z); B.u2n = S(SEG_U2N); B.var = S(SEG_VAR);
     EmitScratch sc;
     T->co.set_levels(g.n_levels);
-    emit_graph(g, B, want_grad, want_marg, T->co, sc);
+    emit_graph(g, B, want_grad, want_marg, want_joint, T->co, sc);
     T->bytes = chunk_bytes(T->co) + 256;
     return T;
 }
@@ -517,7 +525,7 @@ extern "C" int mlbp_plan_compile(int n_graphs, const int32_t *var_off, const int
         mlbp::set_error("plan_compile: bad argument");
         return MLBP_ERR_INVALID;
     }
-    const bool want_grad = flags & 1, want_marg = flags & 2;
+    const bool want_grad = flags & 1, want_marg = flags & 2, want_joint = want_grad && want_marg && (flags & 16);
     const bool prof = std::getenv("MLBP_PLAN_PROFILE") != nullptr;
     auto tnow = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
     double t_a = tnow();
@@ -588,7 +596,7 @@ extern "C" int mlbp_plan_compile(int n_graphs, const int32_t *var_off, const int
                 const int nv = var_off[gi + 1] - var_off[gi], np = pair_off[gi + 1] - pair_off[gi], po = pair_off[gi];
                 const int32_t *r = roots + (size_t)gi * (1 + sweeps);
                 key.clear();
-                key.push_back(nv); key.push_back(np); key.push_back(sweeps); key.push_back(flags & 15);
+                key.push_back(nv); key.push_back(np); key.push_back(sweeps); key.push_back(flags & 31);
                 // r[0] only feeds has_loops (LBP.py:176), whose answer does not depend on the start node when the graph is
                 // connected (create_factor_graph's cliques are): then it is left out of the key (union-find over the factors)
                 int first_root = r[0];
@@ -685,7 +693,8 @@ extern "C" int mlbp_plan_compile(int n_graphs, const int32_t *var_off, const int
                         co.dest[L].reserve(n[4]); co.first[L].reserve(n[5]); co.second[L].reserve(n[6]);
                     }
                     co.init_rows.reserve(flat[0]);
-                    for (auto *v : {&co.pair_c, &co.pair_r, &co.pair_z, &co.pair_u0, &co.pair_u1, &co.pair_u2, &co.pair_g1, &co.pair_gv0, &co.pair_gv1})
+                    for (auto *v : {&co.pair_c, &co.pair_r, &co.pair_z, &co.pair_u0, &co.pair_u1, &co.pair_u2, &co.pair_g1, &co.pair_gv0, &co.pair_gv1,
+                                    &co.pair_m0, &co.pair_m1})
                         v->reserve(flat[1]);
                     co.mu.reserve(flat[2]); co.moff.reserve(flat[3]); co.min_.reserve(flat[4]);
                 }
@@ -717,6 +726,7 @@ extern "C" int mlbp_plan_compile(int n_graphs, const int32_t *var_off, const int
                     append_reloc(co.pair_u0, t.pair_u0, sb); append_reloc(co.pair_u1, t.pair_u1, sb); append_reloc(co.pair_u2, t.pair_u2, sb);
                     co.pair_g1.insert(co.pair_g1.end(), t.pair_g1.begin(), t.pair_g1.end());
                     append_reloc(co.pair_gv0, t.pair_gv0, sb); append_reloc(co.pair_gv1, t.pair_gv1, sb);
+                    append_reloc(co.pair_m0, t.pair_m0, sb); append_reloc(co.pair_m1, t.pair_m1, sb);
                     append_shift(co.moff, t.moff, (int32_t)co.min_.size());
                     append_reloc(co.mu, t.mu, sb);
                     append_reloc(co.min_, t.min_, sb);
@@ -780,7 +790,7 @@ extern "C" int mlbp_plan_compile(int n_graphs, const int32_t *var_off, const int
                 Bases B;
                 B.blk = blk.data();
                 grad_bases(gi, B);
-                emit_graph(G[gi], B, want_grad, want_marg, co, sc);
+                emit_graph(G[gi], B, want_grad, want_marg, want_joint, co, sc);
             }
         });
     }
@@ -892,6 +902,10 @@ extern "C" int mlbp_plan_compile(int n_graphs, const int32_t *var_off, const int
         B[H_MARG_U] = concat([](ChunkOut &x) -> std::vector<int32_t> & { return x.mu; }, false);
         B[H_MARG_OFF] = concat([](ChunkOut &x) -> std::vector<int32_t> & { return x.moff; }, true);
         B[H_MARG_IN] = concat([](ChunkOut &x) -> std::vector<int32_t> & { return x.min_; }, false);
+    }
+    if (want_joint) {                                              // last, so that everything before is the blob without flag bit 4
+        B[H_PAIR_M0] = concat([](ChunkOut &x) -> std::vector<int32_t> & { return x.pair_m0; }, false);
+        B[H_PAIR_M1] = concat([](ChunkOut &x) -> std::vector<int32_t> & { return x.pair_m1; }, false);
     }
     if (pos > 0x7fffff00ull) { delete P; mlbp::set_error("plan_compile: batch too large"); return MLBP_ERR_INVALID; }
     B.resize(pos, 0);

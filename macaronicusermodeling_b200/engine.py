@@ -25,7 +25,8 @@ from . import _lib
 # plan blob header (csrc/plan.cpp)
 (H_NLEVELS, H_LEVELS_OFF, H_INIT_N, H_INIT_OFF, H_NPAIR, H_PAIR_C, H_PAIR_U0, H_PAIR_U1, H_PAIR_U2, H_PAIR_GAP1,
  H_PAIR_V0, H_PAIR_V1, H_NGRAD_GEMM, H_GRAD_GEMM_OFF, H_MARG_N, H_MARG_U, H_MARG_OFF, H_MARG_IN, H_NGRAPHS,
- H_A_ROWS, H_D_ROWS, H_MAX_IN, H_NVARS, H_PAIR_R, H_PAIR_Z, H_MSG_BLK_N, H_MSG_BLK_OFF, H_MSG_ROWS, H_SPK_BLK_N) = range(29)
+ H_A_ROWS, H_D_ROWS, H_MAX_IN, H_NVARS, H_PAIR_R, H_PAIR_Z, H_MSG_BLK_N, H_MSG_BLK_OFF, H_MSG_ROWS, H_SPK_BLK_N, H_PAIR_M0,
+ H_PAIR_M1) = range(31)
 H_WORDS, LEV_WORDS, GEMM_WORDS = 32, 10, 4
 (PLAN_BLOB_WORDS, PLAN_A_ROWS, PLAN_D_ROWS, PLAN_N_LEVELS, PLAN_N_PAIR, PLAN_N_GEMM_ROWS, PLAN_MAX_IN, PLAN_HDR_WORDS,
  PLAN_N_DEAD, PLAN_TMPL_HITS, PLAN_TMPL_MISSES) = range(11)
@@ -226,9 +227,12 @@ class Corpus(object):
 class Result(object):
     """Outputs of one Engine.run: tensors stay on the device until read."""
 
-    def __init__(self, grad, logp, logp_var, top1, rank, beliefs, stats, messages=None, topk=None):
+    def __init__(self, grad, logp, logp_var, top1, rank, beliefs, stats, messages=None, topk=None, logp_joint=None):
         self.grad, self.logp, self.logp_var, self.top1, self.rank, self.beliefs, self.stats = \
             grad, logp, logp_var, top1, rank, beliefs, stats
+        # want_joint: [n_sent] float64, each sentence's joint log-likelihood of its labels, the Bethe estimate at the final
+        # messages (mlbp_joint_logp); -inf where a label has belief 0.  `logp` is the sum of MARGINAL log-probabilities.
+        self.logp_joint = logp_joint
         self.messages = messages     # final pairwise messages (want_messages): see Engine.run
         # want_topk = K: (idx [n_vars, K] int32, prob [n_vars, K] float32, n_ties [n_vars] int32), best first, made on the
         # device by mlbp_topk_rows (VariableNode.get_max_vocab, LBP.py:402-411)
@@ -518,19 +522,22 @@ class Engine(object):
     def _plan_key(corpus, roots, sweeps, flags):
         return (id(corpus), corpus.n_sent, int(corpus.var_off[-1]), int(corpus.pair_off[-1]), int(sweeps), int(flags), roots.tobytes())
 
-    def _plan_flags(self, want_grad, want_marg, approx_inference=False, approx_beliefs=False):
+    def _plan_flags(self, want_grad, want_marg, approx_inference=False, approx_beliefs=False, want_joint=False):
         """mlbp_plan_compile flags of a run() call under the CURRENT theta (the reduced-pass gates of set_theta decide reuse_z)"""
         approx = approx_inference or approx_beliefs
         grad_hi_only = self.grad_a_terms == 1 and self.grad_hi_only_ok and not approx
         two_pass = self.msg_two_pass_ok and not approx
         fold, reuse_z = not approx_inference, (not approx and not grad_hi_only and not two_pass)
-        return (1 if want_grad else 0) | (2 if want_marg else 0) | (0 if fold else 4) | (0 if reuse_z else 8)
+        return (1 if (want_grad or want_joint) else 0) | (2 if want_marg else 0) | (0 if fold else 4) | (0 if reuse_z else 8) | \
+            (16 if want_joint else 0)
 
-    def compile(self, corpus, roots, sweeps, want_grad, want_marg, fold=True, reuse_z=True):
+    def compile(self, corpus, roots, sweeps, want_grad, want_marg, fold=True, reuse_z=True, want_joint=False):
+        """want_joint: plan the gradient stage and the per-factor rows of mlbp_joint_logp (flag bit 4)"""
         roots = np.ascontiguousarray(roots, dtype=np.int32)
         assert roots.shape[0] == corpus.n_sent and roots.shape[1] >= 1 + sweeps, roots.shape
         roots = np.ascontiguousarray(roots[:, :1 + sweeps])
-        flags = (1 if want_grad else 0) | (2 if want_marg else 0) | (0 if fold else 4) | (0 if reuse_z else 8)
+        flags = (1 if (want_grad or want_joint) else 0) | (2 if want_marg else 0) | (0 if fold else 4) | (0 if reuse_z else 8) | \
+            (16 if want_joint else 0)
         pre = self._pre.pop(self._plan_key(corpus, roots, sweeps, flags), None) if self._pre else None
         if pre is not None:                                       # compiled ahead by precompile(): wait for it, take it
             pre[0].join()
@@ -544,7 +551,8 @@ class Engine(object):
         self.plan_template_misses += int(sizes[PLAN_TMPL_MISSES])
         return handle, sizes
 
-    def precompile(self, corpus, roots, sweeps=3, want_grad=True, want_marg=True, approx_inference=False, approx_beliefs=False):
+    def precompile(self, corpus, roots, sweeps=3, want_grad=True, want_marg=True, approx_inference=False, approx_beliefs=False,
+                   want_joint=False):
         """Start compiling the schedule of a LATER run(corpus, roots, ...) call in a background thread (mlbp_plan_compile keeps
         no Python state and ctypes releases the GIL): the roots of the next SGD step do not depend on theta, so the host can
         compile its first micro-batch while it waits for the GPU to finish the current step.  run() picks the plan up when it
@@ -554,7 +562,7 @@ class Engine(object):
         self.drop_precompiled()
         roots = np.ascontiguousarray(roots, dtype=np.int32)
         roots = np.ascontiguousarray(roots[:, :1 + sweeps])
-        flags = self._plan_flags(want_grad, want_marg, approx_inference, approx_beliefs)
+        flags = self._plan_flags(want_grad, want_marg, approx_inference, approx_beliefs, want_joint)
         box = {}
 
         def work():
@@ -575,20 +583,29 @@ class Engine(object):
         self._pre = {}
 
     def run(self, corpus, roots, sweeps=3, want_grad=True, want_marg=True, want_beliefs=False, want_messages=False,
-            approx_inference=False, approx_beliefs=False, topk=100, reduce_into=None, want_topk=0):
+            approx_inference=False, approx_beliefs=False, topk=100, reduce_into=None, want_topk=0, want_joint=False):
         """All sentences of `corpus` (must fit the workspace; use run_many to micro-batch).  `roots`: int
         [n_sent, 1 + sweeps] variable indices local to each sentence (draw 0 = has_loops, LBP.py:176).
         `reduce_into`: optional device tensor of 16 float64 that this call's sums are ADDED to (mlbp_batch_reduce: the
-        vector trainer.Trainer all-reduces)."""
+        vector trainer.Trainer all-reduces).
+        `want_joint`: also Result.logp_joint, the joint log-likelihood of each sentence's labels (Bethe estimate, K9).  It
+        needs the normaliser Z of every pairwise belief, so the gradient-stage rows run as with want_grad; `grad` is still
+        only the unary part unless want_grad.  Needs want_marg and a set_theta(with_grad=True); not defined for the
+        approximate modes (ValueError)."""
         assert self.theta_ee is not None, 'set_theta first'
-        assert not want_grad or self.with_grad_planes
+        if want_joint and (approx_inference or approx_beliefs):
+            raise ValueError('the joint log-likelihood is not defined for the approximate modes (approx_inference / approx_beliefs)')
+        if want_joint and not want_marg:
+            raise ValueError('want_joint needs want_marg: the joint is built around the per-variable log-marginals')
+        grad_stage = want_grad or want_joint
+        assert not grad_stage or self.with_grad_planes
         if corpus.n_sent == 0:                                    # empty batch: nothing to launch
             dev = self.device
             z = lambda *shape, dt=torch.float64: torch.zeros(shape, dtype=dt, device=dev)
             return Result(z(0, 9), z(0), z(0), z(0, dt=torch.int32), z(0, dt=torch.int32),
                           z(0, self.ld, dt=torch.float32) if want_beliefs else None,
                           {'a_rows': 0, 'd_rows': 0, 'levels': 0, 'gemm_rows': 0, 'dead': 0, 'blob_words': 0},
-                          {'v2f': [], 'f2v': []} if want_messages else None)
+                          {'v2f': [], 'f2v': []} if want_messages else None, logp_joint=z(0) if want_joint else None)
         lib = _lib.load()
         # masked (top-K) message rows: the pairwise normaliser Z must come from its own GEMM row of the final messages
         approx = approx_inference or approx_beliefs
@@ -601,7 +618,7 @@ class Engine(object):
         two_pass = self.msg_two_pass_ok and not approx
         msg_one_pass = two_pass and self.msg_one_pass            # message rows as A_hi . B_hi (see __init__)
         handle, sizes = self.compile(corpus, roots, sweeps, want_grad, want_marg, fold=not approx_inference,
-                                     reuse_z=not approx and not grad_hi_only and not two_pass)
+                                     reuse_z=not approx and not grad_hi_only and not two_pass, want_joint=want_joint)
         self.plan_seconds += _time.perf_counter() - t_plan
         try:
             words = int(sizes[PLAN_BLOB_WORDS])
@@ -627,7 +644,7 @@ class Engine(object):
         td = self.theta_ed
         c = lambda name: _p(corpus.dev(name, dev))
         # one-pass gradient rows (A_hi . B_hi) and two-pass message rows both rely on the spike lists of the var->factor kernel
-        one_pass = want_grad and grad_hi_only and self.grad_one_pass_ok and self.grad_a_terms == 1 and self.grad_b_terms == 1 \
+        one_pass = grad_stage and grad_hi_only and self.grad_one_pass_ok and self.grad_a_terms == 1 and self.grad_b_terms == 1 \
             and (self.gemm_impl & 0xff) != 1
         track = two_pass or one_pass
         peak_flag = _p(self._flags, FLAG_PEAK) if track else None
@@ -775,7 +792,12 @@ class Engine(object):
             oc, orr = int(blob[H_PAIR_C]), int(blob[H_PAIR_R])
             rows = torch.cat([bd[oc:oc + n_pair], bd[orr:orr + n_pair]]).long()
             v2f_rows = (A_hi[rows, :V].double() + A_lo[rows, :V].double()) * (2.0 ** -A_SCALE_LOG2)
-        if want_grad and n_pair:
+        if grad_stage and n_pair:
+            if one_pass and not want_grad:
+                # rows run for the joint alone: their spike words go to a copy, so that a gradient-stage row with more spikes
+                # than slots does not switch the later message rows of this theta to three passes (beliefs stay as without it)
+                joint_words = self._flags[:FLAG_COUNTERS].clone()
+                peak_flag = _p(joint_words)
             if one_pass:
                 # spikes of the gradient stage's r rows (two ranges, listed for the AXPY below) and c rows (cells only)
                 for i in range(int(blob[H_MSG_BLK_N]), int(blob[H_SPK_BLK_N])):
@@ -845,6 +867,18 @@ class Engine(object):
                                            _p(aux), _p(cnts), self.tau, self.tau_label, range_log2 + self.half_range_log2,
                                            _p(top1), _p(rank), _p(self._flags, FLAG_COUNTERS)))
                 self.launches += 2
+        logp_joint = None
+        if want_joint:                                            # K9: the Bethe estimate of the joint at the final messages
+            logp_joint = torch.empty(corpus.n_sent, dtype=torch.float64, device=dev)
+            pair_term = torch.empty(max(n_pair, 1), dtype=torch.float64, device=dev)
+            oc, orr, om0, om1 = (int(blob[h]) for h in (H_PAIR_C, H_PAIR_R, H_PAIR_M0, H_PAIR_M1))
+            self._timed('K9 joint_logp', 16.0 * n_pair * V,     # c and r rows (hi + lo fp16), the two mu rows (fp32)
+                        lambda: k.call('mlbp_joint_logp', corpus.n_sent, n_pair, c('var_off'), c('pair_off'), _p(logp_var),
+                                       _p(bd, oc), _p(bd, orr), _p(bd, om0), _p(bd, om1), _p(bd, int(blob[H_PAIR_V0])),
+                                       _p(bd, int(blob[H_PAIR_V1])), c('var_label'), _p(bd, int(blob[H_PAIR_GAP1])),
+                                       _p(pair_stats), _p(A_hi), _p(A_lo), _p(D), ld, V, _p(m.pmi), _p(m.w1), ld,
+                                       _hp(self.theta_ee), -(A_SCALE_LOG2 + self.centre_exp), _p(pair_term), _p(logp_joint)))
+            self.launches += 1
         top_words = None
         if want_marg and want_topk:                               # after the re-score: K5b only moves top1 / rank, not beliefs
             top_words = self.topk_rows(beliefs, min(int(want_topk), V))
@@ -884,7 +918,7 @@ class Engine(object):
         stats = {'a_rows': int(sizes[PLAN_A_ROWS]), 'd_rows': int(sizes[PLAN_D_ROWS]), 'levels': int(sizes[PLAN_N_LEVELS]),
                  'gemm_rows': int(sizes[PLAN_N_GEMM_ROWS]), 'dead': int(sizes[PLAN_N_DEAD]), 'blob_words': words,
                  'msg_two_pass': bool(two_pass), 'msg_passes': 1 if msg_one_pass else (2 if two_pass else 3)}
-        return Result(grad, logp, logp_var, top1, rank, beliefs, stats, messages, top_words)
+        return Result(grad, logp, logp_var, top1, rank, beliefs, stats, messages, top_words, logp_joint)
 
     def topk_rows(self, X, K):
         """the K largest entries of every row of the fp32 device matrix X[:, :V], best first: (idx, value, n_ties) device
@@ -927,7 +961,8 @@ class Engine(object):
         return out
 
     def prepare(self, corpus, sweeps=3, want_grad=True):
-        """Micro-batch slices of `corpus` with their index arrays already resident on the device."""
+        """Micro-batch slices of `corpus` with their index arrays already resident on the device (want_grad: sized for the
+        gradient-stage rows, which run_prepared(want_joint=True) runs too)."""
         parts = []
         for lo, hi in self.microbatches(corpus, sweeps, want_grad):
             c = corpus.slice(lo, hi) if (lo, hi) != (0, corpus.n_sent) else corpus
@@ -937,36 +972,42 @@ class Engine(object):
             parts.append((lo, hi, c))
         return parts
 
-    def run_prepared(self, parts, roots, sweeps=3, want_grad=True, want_marg=True, reduce_into=None, collect=True, **kw):
-        """`collect` = False (with reduce_into): only the batch-level sums are wanted, nothing is concatenated"""
+    def run_prepared(self, parts, roots, sweeps=3, want_grad=True, want_marg=True, reduce_into=None, collect=True,
+                     want_joint=False, **kw):
+        """`collect` = False (with reduce_into): only the batch-level sums are wanted, nothing is concatenated.
+        want_joint: a fifth result, logp_joint [B] (see run)"""
         roots = np.ascontiguousarray(roots, dtype=np.int32)
-        grads, logps, top1s, ranks = [], [], [], []
+        grads, logps, top1s, ranks, joints = [], [], [], [], []
         for lo, hi, c in parts:
-            r = self.run(c, roots[lo:hi], sweeps, want_grad, want_marg, reduce_into=reduce_into, **kw)
+            r = self.run(c, roots[lo:hi], sweeps, want_grad, want_marg, reduce_into=reduce_into, want_joint=want_joint, **kw)
             if not collect:
                 continue
-            grads.append(r.grad); logps.append(r.logp)
+            grads.append(r.grad); logps.append(r.logp); joints.append(r.logp_joint)
             if want_marg:
                 top1s.append(r.top1); ranks.append(r.rank)
-        if not collect:
-            return None, None, None, None
-        cat = lambda xs: xs[0] if len(xs) == 1 else torch.cat(xs)
-        return cat(grads), cat(logps), (cat(top1s) if top1s else None), (cat(ranks) if ranks else None)
+        return self._collected(collect, want_joint, grads, logps, top1s, ranks, joints)
 
-    def run_many(self, corpus, roots, sweeps=3, want_grad=True, want_marg=True, reduce_into=None, collect=True, **kw):
-        """Micro-batched run over a large corpus; returns (grad [B, 9], logp [B], top1 [NV], rank [NV]) on device.
+    @staticmethod
+    def _collected(collect, want_joint, grads, logps, top1s, ranks, joints):
+        out = (None, None, None, None)
+        if collect:
+            cat = lambda xs: xs[0] if len(xs) == 1 else torch.cat(xs)
+            out = (cat(grads), cat(logps), (cat(top1s) if top1s else None), (cat(ranks) if ranks else None))
+        return out + ((cat(joints) if collect else None),) if want_joint else out
+
+    def run_many(self, corpus, roots, sweeps=3, want_grad=True, want_marg=True, reduce_into=None, collect=True,
+                 want_joint=False, **kw):
+        """Micro-batched run over a large corpus; returns (grad [B, 9], logp [B], top1 [NV], rank [NV]) on device, and
+        logp_joint [B] as a fifth entry with want_joint (see run).
         Launches are asynchronous: the host compiles the next micro-batch's schedule while the GPU works."""
         roots = np.ascontiguousarray(roots, dtype=np.int32)
-        grads, logps, top1s, ranks = [], [], [], []
-        for lo, hi in self.microbatches(corpus, sweeps, want_grad):
+        grads, logps, top1s, ranks, joints = [], [], [], [], []
+        for lo, hi in self.microbatches(corpus, sweeps, want_grad or want_joint):
             r = self.run(corpus.slice(lo, hi) if (lo, hi) != (0, corpus.n_sent) else corpus, roots[lo:hi], sweeps,
-                         want_grad, want_marg, reduce_into=reduce_into, **kw)
+                         want_grad, want_marg, reduce_into=reduce_into, want_joint=want_joint, **kw)
             if not collect:
                 continue
-            grads.append(r.grad); logps.append(r.logp)
+            grads.append(r.grad); logps.append(r.logp); joints.append(r.logp_joint)
             if want_marg:
                 top1s.append(r.top1); ranks.append(r.rank)
-        if not collect:
-            return None, None, None, None
-        cat = lambda xs: xs[0] if len(xs) == 1 else torch.cat(xs)
-        return cat(grads), cat(logps), (cat(top1s) if top1s else None), (cat(ranks) if ranks else None)
+        return self._collected(collect, want_joint, grads, logps, top1s, ranks, joints)

@@ -53,6 +53,8 @@ def parse(argv=None):
     opt.add_argument('--report_times', dest='report_times', default=False, action='store_true')
     opt.add_argument('--use_correct_feat', dest='use_correct_feat', default=True, action='store_true')
     opt.add_argument('--seed', dest='seed', type=int, default=1234)                   # train.py:436
+    # not a reference flag: also report each sentence's joint log-likelihood of its labels (Bethe estimate, Engine.run want_joint)
+    opt.add_argument('--joint_likelihood', dest='joint_likelihood', default=False, action='store_true')
     return opt.parse_args(argv)
 
 
@@ -199,13 +201,15 @@ def merge_parts(path, parts, spans):
             os.remove(p)
 
 
-def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None, out_path=None):
+def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None, out_path=None, joint=False):
     """train.py:308-338 batched and sharded over the torchrun ranks.  `units`: prediction_units(); `thetas`: domain ->
     (theta_ee, theta_ed) for the adaptation modes (else the engine's current theta is used).  The roots of every sentence are
     drawn from `rng` in unit order before the units are shared out, so a sentence gets the same roots on any number of ranks.
     Rank r runs units r, r + world, ...; with `out_path` (and not qp) each rank writes its sentences' .pred / .dist text
     to part files next to the output, and after a barrier rank 0 merges them in file order.  Returns the all-reduced
-    (sum log-posterior, (p0, p25, p50, total)) on every rank, summed in the order one process sums them."""
+    (sum log-posterior, (p0, p25, p50, total)) on every rank, summed in the order one process sums them.
+    `joint`: also the sum of the sentences' joint log-likelihoods (Engine.run want_joint) as a third result, and with `out_path`
+    the file <out_path>.joint, one line  sent_id TAB joint TAB sum of marginal logp  per sentence in file order."""
     import torch
     from .engine import Corpus
     from .trainer import dist_info
@@ -213,13 +217,18 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
     V = len(en_domain)
     corpora = [Corpus([sents[i] for i in idx]) for _, idx in units]
     roots = [draw_roots(c, 3, rng) for c in corpora]
-    stats = np.zeros((len(units), 5))                           # per unit: sum logp, #rank == 0, < 26, < 50, variables
+    stats = np.zeros((len(units), 6))                           # per unit: sum logp, #rank == 0, < 26, < 50, variables, sum joint
     write = bool(out_path) and not qp
     if write:
         parts = [out_path + '.rank%d.part' % r for r in range(world)]
         dparts = [out_path + '.dist.rank%d.part' % r for r in range(world)]
         wp, wd = open(parts[rank], 'wb'), open(dparts[rank], 'wb')
         spans, p_off, d_off = [], 0, 0                          # (sentence, .pred offset, length, .dist offset, length)
+    write_joint = bool(out_path) and joint
+    if write_joint:
+        jparts = [out_path + '.joint.rank%d.part' % r for r in range(world)]
+        wj = open(jparts[rank], 'wb')
+        jspans, j_off = [], 0                                   # (sentence, .joint offset, length)
     pinned = [None]
     cur = object()
     for u in range(rank, len(units), world):
@@ -229,9 +238,19 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
             cur = dom
         corpus = corpora[u]
         r = engine.run(corpus, roots[u], 3, want_grad=False, want_marg=True, want_beliefs=not qp,
-                       approx_inference=options.use_approx_inference, want_topk=0 if qp else min(50, V - 1))
+                       approx_inference=options.use_approx_inference, want_topk=0 if qp else min(50, V - 1), want_joint=joint)
         rk = r.rank.cpu().numpy()
-        stats[u] = (float(r.logp.sum().item()), int((rk == 0).sum()), int((rk < 26).sum()), int((rk < 50).sum()), len(rk))
+        stats[u, :5] = (float(r.logp.sum().item()), int((rk == 0).sum()), int((rk < 26).sum()), int((rk < 50).sum()), len(rk))
+        if joint:
+            lj = r.logp_joint.cpu().numpy()
+            stats[u, 5] = float(lj.sum())
+        if write_joint:
+            lm = r.logp.cpu().numpy()
+            for si, i in enumerate(idx):
+                nodes = sorted(raw[i]['current_sent'], key=lambda n: int(n['position']))
+                j_len = wj.write(('%s\t%r\t%r\n' % (nodes[0]['sent_id'], float(lj[si]), float(lm[si]))).encode('utf8'))
+                jspans.append((i, j_off, j_len))
+                j_off += j_len
         if not write:
             continue
         text, toff = dist_text(engine, r.beliefs, pinned)
@@ -289,15 +308,33 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
                     where[i] = (rr, po, pl, do, dl)
             merge_parts(out_path, parts, [(w[0], w[1], w[2]) for w in where])
             merge_parts(out_path + '.dist', dparts, [(w[0], w[3], w[4]) for w in where])
-    logp_sum, k = 0.0, 0
-    while k < len(units):                                       # one partial sum per domain, as the single-process loop
-        part, d = 0.0, units[k][0]
-        while k < len(units) and units[k][0] == d:
-            part += float(stats[k, 0])
-            k += 1
-        logp_sum += part
-    c = stats[:, 1:].sum(axis=0) if len(units) else np.zeros(4)
-    return logp_sum, tuple(int(x) for x in c)
+    if write_joint:
+        wj.close()
+        every = [jspans]
+        if world > 1:
+            every = [None] * world
+            dist.all_gather_object(every, jspans)
+            dist.barrier()
+        if rank == 0:
+            where = [None] * len(sents)
+            for rr, sp in enumerate(every):
+                for i, jo, jl in sp:
+                    where[i] = (rr, jo, jl)
+            merge_parts(out_path + '.joint', jparts, where)
+    sums = []
+    for col in (0, 5):
+        total, k = 0.0, 0
+        while k < len(units):                                   # one partial sum per domain, as the single-process loop
+            part, d = 0.0, units[k][0]
+            while k < len(units) and units[k][0] == d:
+                part += float(stats[k, col])
+                k += 1
+            total += part
+        sums.append(total)
+    c = stats[:, 1:5].sum(axis=0) if len(units) else np.zeros(4)
+    if joint:
+        return sums[0], tuple(int(x) for x in c), sums[1]
+    return sums[0], tuple(int(x) for x in c)
 
 
 def main(argv=None):
@@ -418,12 +455,15 @@ def main(argv=None):
             if tune_lines is not None:
                 engine.set_theta(tr.theta_ee, tr.theta_ed, with_grad=True)
                 tune_sents = lower(tune_lines, options, en2id, de2id)
-                lp, (p0, p25, p50, tot) = predict(engine, prediction_units(len(tune_sents)), tune_sents,
-                                                  [json.loads(l) for l in tune_lines], en_domain, options, rng, True)
+                res = predict(engine, prediction_units(len(tune_sents)), tune_sents, [json.loads(l) for l in tune_lines],
+                              en_domain, options, rng, True, joint=options.joint_likelihood)
+                lp, (p0, p25, p50, tot) = res[:2]
                 if rank == 0:
                     print('\ntune prediction probs:', lp / float(len(tune_lines)))
                     for name, p in (('Prec at 0:', p0), ('prec at 25:', p25), ('prec at 50:', p50)):
                         print(name, '%0.2f' % (float(100 * p) / float(max(tot, 1))), 'total:', tot)
+                    if options.joint_likelihood:
+                        print('tune prediction joint log-likelihood:', res[2] / float(len(tune_lines)))
         print('\ntheta final:', tr.theta_ee, tr.theta_ed)
         if rank == 0 and options.save_params_file:
             save_params(codecs.open(options.save_params_file, 'w', 'utf8'), tr.theta_ee.reshape(1, -1), tr.theta_ed.reshape(1, -1),
@@ -440,12 +480,15 @@ def main(argv=None):
     else:
         engine.set_theta(theta_ee.reshape(-1), theta_ed.reshape(-1), with_grad=True)
         thetas, units = None, prediction_units(len(all_sents))
-    lp, (p0, p25, p50, tot) = predict(engine, units, all_sents, raw, en_domain, options, rng, options.quick_predict, thetas,
-                                      options.save_predictions_file)
+    res = predict(engine, units, all_sents, raw, en_domain, options, rng, options.quick_predict, thetas,
+                  options.save_predictions_file, joint=options.joint_likelihood)
+    lp, (p0, p25, p50, tot) = res[:2]
     if rank == 0:
         print('\nprediction probs:', lp / float(len(train_lines)))
         for name, p in (('Prec at 0:', p0), ('prec at 25:', p25), ('prec at 50:', p50)):
             print(name, '%0.2f' % (float(100 * p) / float(max(tot, 1))), 'total:', tot)
+        if options.joint_likelihood:
+            print('prediction joint log-likelihood:', res[2] / float(len(train_lines)))
     if torch.cuda.is_available():
         torch.cuda.synchronize()
     return 0

@@ -333,6 +333,36 @@ int mlbp_joint_logp(int n_sent, int n_pairs, const int32_t *sent_var_off, const 
                     const double *pair_stats, const void *A_hi, const void *A_lo, const float *D, int ldv, int V,
                     const float *pmi, const float *pmi_w1, int ldf, const double *h_theta_ee, int z_scale_log2,
                     double *pair_term, double *logp_joint, void *stream);
+/* K10. Max-product factor->variable messages (not in the reference, which runs sum-product only): for r < n_rows, n < V
+ *     D[d_row0 + r, n] = max_{k < V} ( a[r, k] / amax_r ) * T'[n, k]
+ *   a[r, k] = (A_hi + A_lo)[a_row0 + r, k] in fp32 (exact), amax_r = max_k a[r, k] (a row with amax_r = 0 gives a zero D row),
+ *   T' the message table `table` (MLBP_TABLE_T, TT, T1 or T1T) in the B[n][k] orientation documented above, formed from the fp32
+ *   feature planes pmi / pmi_w1 [V, ldf]:  T'[a, b] = exp(th[0] pmi[a, b] + [T1, T1T] th[1] pmi_w1[a, b] + th[2] - centre_exp ln 2)
+ *   with K2's compensated argument (~1 ulp; K2's fp16 planes are not read).  Every output lies within [min T', max T'] up to a few
+ *   ulp.  Columns k >= V of A and of the planes are never used; only columns [0, V) of D are written.  fp32 products, exact max:
+ *   bit-identical for any row slicing.  Needs ldv % 8 == 0, ldf % 4 == 0 and 16-byte aligned A_hi, A_lo, pmi, pmi_w1.
+ *   MLBP_ERR_INVALID, nothing launched: a null pointer, an unknown table id, V < 1, ldv / ldf / ldd < V, a row range outside
+ *   [0, a_rows_total), the alignment above.  n_rows == 0 is a no-op.                                                             */
+int mlbp_factor_to_var_maxprod(const void *A_hi, const void *A_lo, int64_t a_rows_total, int a_row0, int n_rows, int table,
+                               const float *pmi, const float *pmi_w1, int V, int ldv, int ldf, const double *h_theta_ee,
+                               int centre_exp, float *D, int64_t d_row0, int ldd, void *stream);
+/* K11. Log of the unnormalised joint potential of an assignment x (one int32 word per variable, sentence s owns variables
+ *   [var_off[s], var_off[s + 1])), float64 per sentence (the model of SURVEY.md Appendix A; train.py:218-253, :255-297):
+ *     score[s] = sum_{i in s} [ td[0] edT[d_i, x_i] + td[1] pedT[d_i, x_i] + td[5]
+ *                               + sum over the sparse features (e, f, val) of i with e == x_i of td[f] val
+ *                               + sum over the given tokens j of i of l_{gap1}(x_i, giv_label[j]) ]
+ *              + sum over the pairwise factors (v0, v1) of s (pair indices local to the sentence) of l_{gap1}(x_v0, x_v1)
+ *     l_g(a, b) = te[0] pmi[a, b] + te[2] + g te[1] pmi_w1[a, b]
+ *   (no en_de term where var_de < 0).  Corpus arrays as in mlbp_unary_stats / mlbp_plan_compile; pmi, pmi_w1 [V, ldf] and edT,
+ *   pedT [Vd, ldf] fp32.  One warp per sentence, fixed summation order (deterministic).  n_vars = var_off[n_sent] and n_given =
+ *   giv_off[n_vars] are checked, and so is every x[i] and giv_label[j] against [0, V): on the host, after a copy that
+ *   SYNCHRONISES the stream; MLBP_ERR_INVALID, nothing launched.                                                                */
+int mlbp_assignment_score(int n_sent, int n_vars, int n_given, const int32_t *var_off, const int32_t *x, const int32_t *var_de,
+                          const int32_t *sp_off, const int32_t *sp_en, const int32_t *sp_feat, const float *sp_val,
+                          const int32_t *giv_off, const int32_t *giv_label, const int32_t *giv_gap1, const int32_t *pair_off,
+                          const int32_t *pair_v0, const int32_t *pair_v1, const int32_t *pair_gap1, const float *pmi,
+                          const float *pmi_w1, const float *edT, const float *pedT, int V, int ldf, const double *h_theta_ee,
+                          const double *h_theta_ed, double *score, void *stream);
 /* rows[0] = 1.0f (the constant-one row the kernels read for a message that is still uniform), rows[1 + t] = the message of a
  *   pairwise factor of message table t (MLBP_TABLE_T .. T1T) that is fed the uniform initial message (LBP.py:211-216 +
  *   :509 / :518): the row / column sums of the table, mean-one scaled.  rows: [MLBP_D_CONST_ROWS, ldv] fp32; the engine

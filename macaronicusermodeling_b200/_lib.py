@@ -35,6 +35,8 @@ _SIGNATURES = {
     'mlbp_batch_reduce': 'ippipppp',
     'mlbp_const_rows': 'piipp',
     'mlbp_joint_logp': 'ii' + 'ppp' + 'pppp' + 'pppp' + 'ppppii' + 'ppi' + 'pi' + 'pp' + 'p',
+    'mlbp_factor_to_var_maxprod': 'ppliii' + 'ppiii' + 'pi' + 'pli' + 'p',
+    'mlbp_assignment_score': 'iii' + 'pppppppp' + 'pppppppp' + 'pp' + 'ii' + 'ppp' + 'p',
     'mlbp_plan_compile': 'ipppppp' + 'iip',
     'mlbp_plan_sizes': 'pp',
     'mlbp_plan_export': 'pp',

@@ -45,6 +45,31 @@ __device__ __forceinline__ void split_f16(float x, __half &hi, __half &lo) {
     lo = __float2half_rn(x - __half2float(hi));
 }
 
+// Compensated fp32 arithmetic of the table entries exp(theta . phi) (K2, K10): ~1 ulp of fp32 per entry without a float64
+// instruction per element.
+struct F2 { float hi, lo; };                                      // unevaluated sum hi + lo
+
+__host__ __device__ __forceinline__ F2 split_double(double x) {
+    F2 r;
+    r.hi = (float)x;
+    r.lo = (float)(x - (double)r.hi);
+    return r;
+}
+// c * p + b with c = (c.hi + c.lo), b = (b.hi + b.lo), p an fp32 datum: result as hi + lo (error ~2^-46 relative)
+__device__ __forceinline__ F2 axpb(F2 c, float p, F2 b) {
+    const float ph = c.hi * p;
+    const float pe = fmaf(c.hi, p, -ph);                          // exact product error
+    const float s = ph + b.hi;
+    const float bb = s - ph;
+    const float se = (ph - (s - bb)) + (b.hi - bb);               // exact sum error (two-sum)
+    F2 r;
+    r.hi = s;
+    r.lo = se + pe + fmaf(c.lo, p, b.lo);
+    return r;
+}
+// exp(z.hi + z.lo), ~1 ulp: expf is IEEE-grade here (the library is built without fast-math)
+__device__ __forceinline__ float exp_f2(F2 z) { return expf(z.hi) * (1.0f + z.lo); }
+
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

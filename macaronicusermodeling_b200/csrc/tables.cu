@@ -19,32 +19,6 @@ constexpr int TS = 64;  // tile edge
 struct ThetaEE { double pmi, w1, bias; };
 struct ThetaED { double t[6]; };
 
-struct F2 { float hi, lo; };                                      // unevaluated sum hi + lo
-
-__device__ __forceinline__ F2 split_double(double x) {
-    F2 r;
-    r.hi = (float)x;
-    r.lo = (float)(x - (double)r.hi);
-    return r;
-}
-// c * p + b with c = (c.hi + c.lo), b = (b.hi + b.lo), p an fp32 datum: result as hi + lo (error ~2^-46 relative)
-__device__ __forceinline__ F2 axpb(F2 c, float p, F2 b) {
-    const float ph = c.hi * p;
-    const float pe = fmaf(c.hi, p, -ph);                          // exact product error
-    const float s = ph + b.hi;
-    const float bb = s - ph;
-    const float se = (ph - (s - bb)) + (b.hi - bb);               // exact sum error (two-sum)
-    F2 r;
-    r.hi = s;
-    r.lo = se + pe + fmaf(c.lo, p, b.lo);
-    return r;
-}
-static F2 split_double_host(double x) {
-    F2 r;
-    r.hi = (float)x;
-    r.lo = (float)(x - (double)r.hi);
-    return r;
-}
 // s += x for an unevaluated sum s = (hi, lo): two-sum, the rounding error of every addition is kept in lo
 __device__ __forceinline__ void acc_f2(F2 &s, float x) {
     const float t = s.hi + x;
@@ -73,9 +47,6 @@ __device__ __forceinline__ __half half_stochastic_signed(float x, unsigned r) { 
     const __half h = half_stochastic(fabsf(x), r);
     return x < 0.f ? __hneg(h) : h;
 }
-
-// exp(z.hi + z.lo), ~1 ulp: expf is IEEE-grade here (the library is built without fast-math)
-__device__ __forceinline__ float exp_f2(F2 z) { return expf(z.hi) * (1.0f + z.lo); }
 
 // One 64x64 tile of the (a, b) plane per CTA, 256 threads: thread (tx = tid % 32, ty = tid / 32) owns the column pair
 // b0 + 2 tx, + 1 of rows ty, ty + 8, ...: 8-byte global loads and 4-byte (half2) plane stores, 128 bytes per warp and plane.
@@ -254,8 +225,8 @@ extern "C" int mlbp_build_pairwise_tables(const float *pmi, const float *pmi_w1,
                                        12 * TS * (TS + 2) * (int)sizeof(__half)));
         attr_set_dev[current_device()] = true;
     }
-    build_pairwise_tables_kernel<<<grid, 256, smem, st>>>(pmi, pmi_w1, V, ldf, split_double_host(h_theta_ee[0]),
-                                                       split_double_host(h_theta_ee[1]), split_double_host(h_theta_ee[2]),
+    build_pairwise_tables_kernel<<<grid, 256, smem, st>>>(pmi, pmi_w1, V, ldf, split_double(h_theta_ee[0]),
+                                                       split_double(h_theta_ee[1]), split_double(h_theta_ee[2]),
                                                        ldexpf(1.0f, scale_exp), (__half *)planes, plane_stride, ldv, colsums,
                                                        with_grad_planes, (__half *)r_planes, tbar);
     MLBP_LAUNCH_CHECK();

@@ -227,12 +227,16 @@ class Corpus(object):
 class Result(object):
     """Outputs of one Engine.run: tensors stay on the device until read."""
 
-    def __init__(self, grad, logp, logp_var, top1, rank, beliefs, stats, messages=None, topk=None, logp_joint=None):
+    def __init__(self, grad, logp, logp_var, top1, rank, beliefs, stats, messages=None, topk=None, logp_joint=None,
+                 map_score=None, label_score=None):
         self.grad, self.logp, self.logp_var, self.top1, self.rank, self.beliefs, self.stats = \
             grad, logp, logp_var, top1, rank, beliefs, stats
         # want_joint: [n_sent] float64, each sentence's joint log-likelihood of its labels, the Bethe estimate at the final
         # messages (mlbp_joint_logp); -inf where a label has belief 0.  `logp` is the sum of MARGINAL log-probabilities.
         self.logp_joint = logp_joint
+        # max_product: [n_sent] float64, the log of the unnormalised joint potential of the decoded assignment (top1) and of the
+        # labels (mlbp_assignment_score); map_score - label_score is the log-odds of the model's best joint guess against the labels
+        self.map_score, self.label_score = map_score, label_score
         self.messages = messages     # final pairwise messages (want_messages): see Engine.run
         # want_topk = K: (idx [n_vars, K] int32, prob [n_vars, K] float32, n_ties [n_vars] int32), best first, made on the
         # device by mlbp_topk_rows (VariableNode.get_max_vocab, LBP.py:402-411)
@@ -319,6 +323,8 @@ class Engine(object):
         self.planes = None
         self.colsums = torch.zeros((N_SUMS, self.V), dtype=torch.float64, device=self.device)
         self.const_rows = None      # factor->variable messages of a pairwise factor fed the uniform initial message
+        self.map_const_rows = None  # the same for max-product messages (K10), built on first use after each set_theta
+        self.map_const_ok = False
         self.edstats = torch.zeros((self.Vd, 3), dtype=torch.float64, device=self.device)
         self.with_grad_planes = False
         self._A = self._D = self._U = None
@@ -424,6 +430,35 @@ class Engine(object):
             self.const_rows = torch.empty((D_CONST_ROWS, self.ld), dtype=torch.float32, device=self.device)
         self.k.call('mlbp_const_rows', _p(self.colsums), self.V, self.ld, _p(self.const_rows))
         self.launches += 1
+        self.map_const_ok = False
+
+    def maxprod_rows(self, A_hi, A_lo, a_rows_total, a_row0, n_rows, table, D, d_row0):
+        """K10: max-product factor->variable messages of A rows [a_row0, a_row0 + n_rows) into D rows d_row0 .. under the current
+        theta, row-normalised by each row's max and centred like the sum-product rows (mlbp_factor_to_var_maxprod)"""
+        m = self.model
+        self._timed('K10 maxprod', lambda: n_rows * self.V * 8.0 + (2 if table in (2, 3) else 1) * self.V * self.V * 4.0,
+                    lambda: self.k.call('mlbp_factor_to_var_maxprod', _p(A_hi), _p(A_lo), int(a_rows_total), int(a_row0),
+                                        int(n_rows), int(table), _p(m.pmi), _p(m.w1), self.V, self.ld, self.ld,
+                                        _hp(self.theta_ee), self.centre_exp, _p(D), int(d_row0), int(D.shape[1])))
+        self.launches += 1
+
+    def _map_const(self):
+        """D rows 0..4 of a max-product run: the constant-one row and, per message table, K10 of the uniform message -- the row
+        (T, T1) or column (Tt, T1t) maxima of the centred table"""
+        if self.map_const_ok:
+            return self.map_const_rows
+        if self.map_const_rows is None:
+            self.map_const_rows = torch.zeros((D_CONST_ROWS, self.ld), dtype=torch.float32, device=self.device)
+            self._map_uniform = torch.zeros((2, 1, self.ld), dtype=torch.float16, device=self.device)
+            rows = torch.zeros(1, dtype=torch.int32, device=self.device)
+            self.k.call('mlbp_fill_uniform_rows', _p(self._map_uniform[0]), _p(self._map_uniform[1]), self.ld, self.V, _p(rows), 1,
+                        None)
+            self.launches += 1
+        self.map_const_rows[0].copy_(self.const_rows[0])
+        for t in range(4):
+            self.maxprod_rows(self._map_uniform[0], self._map_uniform[1], 1, 0, 1, t, self.map_const_rows, 1 + t)
+        self.map_const_ok = True
+        return self.map_const_rows
 
     def pass_stats(self):
         """Host copy of the device-side decisions since the last set_theta (one small D2H read): whether a peaked message
@@ -583,7 +618,8 @@ class Engine(object):
         self._pre = {}
 
     def run(self, corpus, roots, sweeps=3, want_grad=True, want_marg=True, want_beliefs=False, want_messages=False,
-            approx_inference=False, approx_beliefs=False, topk=100, reduce_into=None, want_topk=0, want_joint=False):
+            approx_inference=False, approx_beliefs=False, topk=100, reduce_into=None, want_topk=0, want_joint=False,
+            max_product=False):
         """All sentences of `corpus` (must fit the workspace; use run_many to micro-batch).  `roots`: int
         [n_sent, 1 + sweeps] variable indices local to each sentence (draw 0 = has_loops, LBP.py:176).
         `reduce_into`: optional device tensor of 16 float64 that this call's sums are ADDED to (mlbp_batch_reduce: the
@@ -591,8 +627,17 @@ class Engine(object):
         `want_joint`: also Result.logp_joint, the joint log-likelihood of each sentence's labels (Bethe estimate, K9).  It
         needs the normaliser Z of every pairwise belief, so the gradient-stage rows run as with want_grad; `grad` is still
         only the unary part unless want_grad.  Needs want_marg and a set_theta(with_grad=True); not defined for the
-        approximate modes (ValueError)."""
+        approximate modes (ValueError).
+        `max_product`: max-product BP instead of sum-product (K10 replaces every pairwise message row, on the same plan).
+        `top1` is then the decoded assignment -- the arg-max of each variable's max-marginal, first index on ties --, and
+        `beliefs`, `logp_var`, `logp` and `rank` are K5's usual outputs computed on the normalised MAX-marginals.
+        Result.map_score / label_score: the log-potential of the decoded assignment and of the labels (K11).  Inference only:
+        ValueError with want_grad, want_joint, the approximate modes or without want_marg.  Synchronises the stream (K11
+        checks the assignments on the host)."""
         assert self.theta_ee is not None, 'set_theta first'
+        if max_product and (want_grad or want_joint or approx_inference or approx_beliefs or not want_marg):
+            raise ValueError('max_product is inference only: it needs want_marg and does not combine with want_grad, want_joint '
+                             'or the approximate modes (approx_inference / approx_beliefs)')
         if want_joint and (approx_inference or approx_beliefs):
             raise ValueError('the joint log-likelihood is not defined for the approximate modes (approx_inference / approx_beliefs)')
         if want_joint and not want_marg:
@@ -605,7 +650,8 @@ class Engine(object):
             return Result(z(0, 9), z(0), z(0), z(0, dt=torch.int32), z(0, dt=torch.int32),
                           z(0, self.ld, dt=torch.float32) if want_beliefs else None,
                           {'a_rows': 0, 'd_rows': 0, 'levels': 0, 'gemm_rows': 0, 'dead': 0, 'blob_words': 0},
-                          {'v2f': [], 'f2v': []} if want_messages else None, logp_joint=z(0) if want_joint else None)
+                          {'v2f': [], 'f2v': []} if want_messages else None, logp_joint=z(0) if want_joint else None,
+                          map_score=z(0) if max_product else None, label_score=z(0) if max_product else None)
         lib = _lib.load()
         # masked (top-K) message rows: the pairwise normaliser Z must come from its own GEMM row of the final messages
         approx = approx_inference or approx_beliefs
@@ -639,6 +685,9 @@ class Engine(object):
             self._blob_event.record()
         bd = self._blob_dev
         dev, ld, V, k, m = self.device, self.ld, self.V, self.k, self.model
+        if max_product:
+            # the spike scan and compensation, the device gates and the K5b re-score exist only to make reduced-pass GEMM rows safe
+            two_pass = msg_one_pass = False
         A_hi, A_lo, D, U = self._A[0], self._A[1], self._D, self._U
         a_cap = int(self._A.shape[1])
         td = self.theta_ed
@@ -661,7 +710,7 @@ class Engine(object):
             k.call('mlbp_zero_words', _p(spk_blk), max(n_blk, 1))
             k.call('mlbp_zero_words', _p(self._flags, FLAG_NSPIKY), 1)
 
-        D[:D_CONST_ROWS].copy_(self.const_rows)                   # row 0: the constant-one row messages still uniform read
+        D[:D_CONST_ROWS].copy_(self._map_const() if max_product else self.const_rows)   # row 0: the constant-one row
         inv_sigma = torch.empty(max(nv, 1), dtype=torch.float64, device=dev)
         g_unary = torch.empty((max(nv, 1), 9), dtype=torch.float64, device=dev)
         k.call('mlbp_unary_stats', nv, c('var_de'), c('var_label'), c('sp_off'), c('sp_en'), c('sp_feat'), c('sp_val'),
@@ -776,7 +825,12 @@ class Engine(object):
                     t, a0, d0, rows = (int(x) for x in blob[int(rec[7]) + GEMM_WORDS * i: int(rec[7]) + GEMM_WORDS * (i + 1)])
                     if two_pass:
                         spike_scan(a0, rows)
-            if two_pass:
+            if max_product:
+                for i in range(int(rec[6])):
+                    t, a0, d0, rows = (int(x) for x in blob[int(rec[7]) + GEMM_WORDS * i: int(rec[7]) + GEMM_WORDS * (i + 1)])
+                    self.maxprod_rows(A_hi, A_lo, a_cap, a0, rows, t, D, d0)
+                    self.gemm_rows += rows
+            elif two_pass:
                 gemm_calls(int(rec[7]), int(rec[6]), False, GEMM_A_HI_ONLY | (GEMM_B_HI_ONLY if msg_one_pass else 0), gated=True,
                            residual=msg_residual)
                 for i in range(int(rec[6])):                      # restore what the dropped lo half of the spikes contributed
@@ -879,6 +933,18 @@ class Engine(object):
                                        _p(pair_stats), _p(A_hi), _p(A_lo), _p(D), ld, V, _p(m.pmi), _p(m.w1), ld,
                                        _hp(self.theta_ee), -(A_SCALE_LOG2 + self.centre_exp), _p(pair_term), _p(logp_joint)))
             self.launches += 1
+        map_score = label_score = None
+        if max_product:                                           # K11 on the decoded assignment and on the labels
+            map_score = torch.empty(corpus.n_sent, dtype=torch.float64, device=dev)
+            label_score = torch.empty(corpus.n_sent, dtype=torch.float64, device=dev)
+            for x, out in ((_p(top1), map_score), (c('var_label'), label_score)):
+                self._timed('K11 assignment_score', 4.0 * (nv + len(corpus.giv_label) + 2 * corpus.n_pairs),
+                            lambda x=x, out=out: k.call('mlbp_assignment_score', corpus.n_sent, nv, len(corpus.giv_label),
+                                                        c('var_off'), x, c('var_de'), c('sp_off'), c('sp_en'), c('sp_feat'),
+                                                        c('sp_val'), c('giv_off'), c('giv_label'), c('giv_gap1'), c('pair_off'),
+                                                        c('pair_v0'), c('pair_v1'), c('pair_gap1'), _p(m.pmi), _p(m.w1),
+                                                        _p(m.edT), _p(m.pedT), V, ld, _hp(self.theta_ee), _hp(td), _p(out)))
+                self.launches += 1
         top_words = None
         if want_marg and want_topk:                               # after the re-score: K5b only moves top1 / rank, not beliefs
             top_words = self.topk_rows(beliefs, min(int(want_topk), V))
@@ -918,7 +984,7 @@ class Engine(object):
         stats = {'a_rows': int(sizes[PLAN_A_ROWS]), 'd_rows': int(sizes[PLAN_D_ROWS]), 'levels': int(sizes[PLAN_N_LEVELS]),
                  'gemm_rows': int(sizes[PLAN_N_GEMM_ROWS]), 'dead': int(sizes[PLAN_N_DEAD]), 'blob_words': words,
                  'msg_two_pass': bool(two_pass), 'msg_passes': 1 if msg_one_pass else (2 if two_pass else 3)}
-        return Result(grad, logp, logp_var, top1, rank, beliefs, stats, messages, top_words, logp_joint)
+        return Result(grad, logp, logp_var, top1, rank, beliefs, stats, messages, top_words, logp_joint, map_score, label_score)
 
     def topk_rows(self, X, K):
         """the K largest entries of every row of the fp32 device matrix X[:, :V], best first: (idx, value, n_ties) device

@@ -55,6 +55,8 @@ def parse(argv=None):
     opt.add_argument('--seed', dest='seed', type=int, default=1234)                   # train.py:436
     # not a reference flag: also report each sentence's joint log-likelihood of its labels (Bethe estimate, Engine.run want_joint)
     opt.add_argument('--joint_likelihood', dest='joint_likelihood', default=False, action='store_true')
+    # not a reference flag: also decode each sentence's most probable joint guess (max-product BP, Engine.run max_product)
+    opt.add_argument('--map_decode', dest='map_decode', default=False, action='store_true')
     return opt.parse_args(argv)
 
 
@@ -201,7 +203,7 @@ def merge_parts(path, parts, spans):
             os.remove(p)
 
 
-def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None, out_path=None, joint=False):
+def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None, out_path=None, joint=False, map_decode=False):
     """train.py:308-338 batched and sharded over the torchrun ranks.  `units`: prediction_units(); `thetas`: domain ->
     (theta_ee, theta_ed) for the adaptation modes (else the engine's current theta is used).  The roots of every sentence are
     drawn from `rng` in unit order before the units are shared out, so a sentence gets the same roots on any number of ranks.
@@ -209,7 +211,10 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
     to part files next to the output, and after a barrier rank 0 merges them in file order.  Returns the all-reduced
     (sum log-posterior, (p0, p25, p50, total)) on every rank, summed in the order one process sums them.
     `joint`: also the sum of the sentences' joint log-likelihoods (Engine.run want_joint) as a third result, and with `out_path`
-    the file <out_path>.joint, one line  sent_id TAB joint TAB sum of marginal logp  per sentence in file order."""
+    the file <out_path>.joint, one line  sent_id TAB joint TAB sum of marginal logp  per sentence in file order.
+    `map_decode`: every unit also runs max-product inference with the same roots (no further draws from `rng`); one more result
+    (tokens whose decoded word is the label, sentences decoded entirely right), and with `out_path` the file <out_path>.map, one
+    line  sent_id TAB decoded words in position order TAB map_score TAB label_score  per sentence in file order."""
     import torch
     from .engine import Corpus
     from .trainer import dist_info
@@ -217,7 +222,8 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
     V = len(en_domain)
     corpora = [Corpus([sents[i] for i in idx]) for _, idx in units]
     roots = [draw_roots(c, 3, rng) for c in corpora]
-    stats = np.zeros((len(units), 6))                           # per unit: sum logp, #rank == 0, < 26, < 50, variables, sum joint
+    # per unit: sum logp, #rank == 0, < 26, < 50, variables, sum joint, MAP tokens right, MAP sentences right
+    stats = np.zeros((len(units), 8))
     write = bool(out_path) and not qp
     if write:
         parts = [out_path + '.rank%d.part' % r for r in range(world)]
@@ -229,6 +235,11 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
         jparts = [out_path + '.joint.rank%d.part' % r for r in range(world)]
         wj = open(jparts[rank], 'wb')
         jspans, j_off = [], 0                                   # (sentence, .joint offset, length)
+    write_map = bool(out_path) and map_decode
+    if write_map:
+        mparts = [out_path + '.map.rank%d.part' % r for r in range(world)]
+        wm = open(mparts[rank], 'wb')
+        mspans, m_off = [], 0                                   # (sentence, .map offset, length)
     pinned = [None]
     cur = object()
     for u in range(rank, len(units), world):
@@ -251,6 +262,20 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
                 j_len = wj.write(('%s\t%r\t%r\n' % (nodes[0]['sent_id'], float(lj[si]), float(lm[si]))).encode('utf8'))
                 jspans.append((i, j_off, j_len))
                 j_off += j_len
+        if map_decode:
+            rm = engine.run(corpus, roots[u], 3, want_grad=False, want_marg=True, max_product=True)
+            dec, lab = rm.top1.cpu().numpy(), corpus.var_label
+            ok = dec == lab
+            stats[u, 6] = int(ok.sum())
+            stats[u, 7] = sum(1 for si in range(len(idx)) if ok[corpus.var_off[si]:corpus.var_off[si + 1]].all())
+            if write_map:
+                ms, ls = rm.map_score.cpu().numpy(), rm.label_score.cpu().numpy()
+                for si, i in enumerate(idx):
+                    nodes = sorted(raw[i]['current_sent'], key=lambda n: int(n['position']))
+                    words = ' '.join(en_domain[int(e)] for e in dec[corpus.var_off[si]:corpus.var_off[si + 1]])
+                    m_len = wm.write(('%s\t%s\t%r\t%r\n' % (nodes[0]['sent_id'], words, float(ms[si]), float(ls[si]))).encode('utf8'))
+                    mspans.append((i, m_off, m_len))
+                    m_off += m_len
         if not write:
             continue
         text, toff = dist_text(engine, r.beliefs, pinned)
@@ -321,6 +346,19 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
                 for i, jo, jl in sp:
                     where[i] = (rr, jo, jl)
             merge_parts(out_path + '.joint', jparts, where)
+    if write_map:
+        wm.close()
+        every = [mspans]
+        if world > 1:
+            every = [None] * world
+            dist.all_gather_object(every, mspans)
+            dist.barrier()
+        if rank == 0:
+            where = [None] * len(sents)
+            for rr, sp in enumerate(every):
+                for i, mo, ml in sp:
+                    where[i] = (rr, mo, ml)
+            merge_parts(out_path + '.map', mparts, where)
     sums = []
     for col in (0, 5):
         total, k = 0.0, 0
@@ -332,9 +370,19 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
             total += part
         sums.append(total)
     c = stats[:, 1:5].sum(axis=0) if len(units) else np.zeros(4)
+    out = (sums[0], tuple(int(x) for x in c))
     if joint:
-        return sums[0], tuple(int(x) for x in c), sums[1]
-    return sums[0], tuple(int(x) for x in c)
+        out += (sums[1],)
+    if map_decode:
+        out += (tuple(int(x) for x in stats[:, 6:8].sum(axis=0)),)
+    return out
+
+
+def print_map(prefix, counts, n_tokens, n_sents):
+    """the two --map_decode lines: decoded word == label over predicted tokens (compare P@0), and whole sentences right"""
+    print(prefix + 'prediction MAP token accuracy:', '%0.2f' % (float(100 * counts[0]) / float(max(n_tokens, 1))), 'total:', n_tokens)
+    print(prefix + 'prediction MAP sentence accuracy:', '%0.2f' % (float(100 * counts[1]) / float(max(n_sents, 1))), 'total:',
+          n_sents)
 
 
 def main(argv=None):
@@ -346,6 +394,10 @@ def main(argv=None):
         return 1
     if options.user_adapt and options.experience_adapt:
         sys.stderr.write('Currently only supports 1 type of adaptation.')                  # train.py:489-491
+        return 1
+    if options.map_decode and (options.use_approx_inference or options.use_approx_beliefs):
+        sys.stderr.write('--map_decode decodes with exact max-product inference: it does not combine with --use_approx_inference '
+                         'or --use_approx_beliefs\n')
         return 1
     adapt = options.user_adapt or options.experience_adapt
     import os
@@ -456,7 +508,7 @@ def main(argv=None):
                 engine.set_theta(tr.theta_ee, tr.theta_ed, with_grad=True)
                 tune_sents = lower(tune_lines, options, en2id, de2id)
                 res = predict(engine, prediction_units(len(tune_sents)), tune_sents, [json.loads(l) for l in tune_lines],
-                              en_domain, options, rng, True, joint=options.joint_likelihood)
+                              en_domain, options, rng, True, joint=options.joint_likelihood, map_decode=options.map_decode)
                 lp, (p0, p25, p50, tot) = res[:2]
                 if rank == 0:
                     print('\ntune prediction probs:', lp / float(len(tune_lines)))
@@ -464,6 +516,8 @@ def main(argv=None):
                         print(name, '%0.2f' % (float(100 * p) / float(max(tot, 1))), 'total:', tot)
                     if options.joint_likelihood:
                         print('tune prediction joint log-likelihood:', res[2] / float(len(tune_lines)))
+                    if options.map_decode:
+                        print_map('tune ', res[-1], tot, len(tune_sents))
         print('\ntheta final:', tr.theta_ee, tr.theta_ed)
         if rank == 0 and options.save_params_file:
             save_params(codecs.open(options.save_params_file, 'w', 'utf8'), tr.theta_ee.reshape(1, -1), tr.theta_ed.reshape(1, -1),
@@ -481,7 +535,7 @@ def main(argv=None):
         engine.set_theta(theta_ee.reshape(-1), theta_ed.reshape(-1), with_grad=True)
         thetas, units = None, prediction_units(len(all_sents))
     res = predict(engine, units, all_sents, raw, en_domain, options, rng, options.quick_predict, thetas,
-                  options.save_predictions_file, joint=options.joint_likelihood)
+                  options.save_predictions_file, joint=options.joint_likelihood, map_decode=options.map_decode)
     lp, (p0, p25, p50, tot) = res[:2]
     if rank == 0:
         print('\nprediction probs:', lp / float(len(train_lines)))
@@ -489,6 +543,8 @@ def main(argv=None):
             print(name, '%0.2f' % (float(100 * p) / float(max(tot, 1))), 'total:', tot)
         if options.joint_likelihood:
             print('prediction joint log-likelihood:', res[2] / float(len(train_lines)))
+        if options.map_decode:
+            print_map('', res[-1], tot, len(all_sents))
     if torch.cuda.is_available():
         torch.cuda.synchronize()
     return 0

@@ -363,6 +363,45 @@ int mlbp_assignment_score(int n_sent, int n_vars, int n_given, const int32_t *va
                           const int32_t *pair_v0, const int32_t *pair_v1, const int32_t *pair_gap1, const float *pmi,
                           const float *pmi_w1, const float *edT, const float *pedT, int V, int ldf, const double *h_theta_ee,
                           const double *h_theta_ed, double *score, void *stream);
+/* K12. Gibbs sampler of each sentence's joint guesses (not in the reference): for n_sent sentences (variables [var_off[s],
+ *   var_off[s + 1]), k of them, pairwise factors [pair_off[s], ..) with local pair_v0 / pair_v1 as in mlbp_plan_compile; any pair
+ *   list with each pair of variables at most once) and `chains` chains each, the target is
+ *     p(x) ~ prod_i U_i(x_i) * prod_(a, b) T_g(x_a, x_b)      (U: K1's rows [n_vars, ldv] fp32; T_g = T, or T1 where pair_gap1)
+ *   One CTA of MLBP_GIBBS_THREADS threads per (sentence, chain), no inter-CTA communication.  Sweep 0 draws every x_i from U_i
+ *   alone, sweeps 1 .. burn_in are discarded, sweeps burn_in + 1 .. burn_in + n_keep are kept; a sweep updates i = 0 .. k - 1.
+ *   Conditional of i, for x < V:  q(x) = U_i[x], then for every factor touching i in pair-list order
+ *     q = q * ((hi + lo) * f)       hi + lo, (hi + lo) * f and the product each rounded to fp32;
+ *     i dim 0 of (i, b): row x_b of the TT / T1T planes, f = fp32(2^-scale_exp * V / colsums[0 / 1][x_b])  (column sums);
+ *     i dim 1 of (a, i): row x_a of the T / T1 planes,   f = fp32(2^-scale_exp * V / colsums[5 / 6][x_a])  (row sums),
+ *   the mean-one factor K1 applies to a given token.  range_log2 (a bound on |log2| of any such product, as for K3) outside
+ *   [0, 100): the same order in fp64, q = q * (double(hi + lo) * double(f)).
+ *   Draw: E = 8 ceil(V / (8 MLBP_GIBBS_THREADS)); thread t owns columns [t E, t E + E) (q = 0 from V on).  s_t(e) = float64 running
+ *   sum of q over t's columns up to e; S_t = s_t(last); inside each warp an inclusive Kogge-Stone scan of S_t (step d = 1 .. 16:
+ *   v += v of lane - d), its exclusive value E_t (lane 0: 0); O_w = the warp totals of warps < w added in warp order from 0;
+ *   C(e) = (O_w + E_t) + s_t(e); x_i = the smallest x < V with C(x) > u * C(V - 1) (if none: the largest x with q(x) > 0).
+ *   C(V - 1) <= 0 or not finite: x_i = floor(u V) and the Rao-Blackwell term below is fp32(1 / V).
+ *   u = ((w0 >> 5) 2^26 + (w1 >> 6)) 2^-53 with (w0, w1, ..) = Philox4x32-10(counter (sent_id[s], chain, sweep, i), key
+ *   (seed & 0xffffffff, seed >> 32)): a sentence's chain does not depend on its batch, its position or the launch.
+ *   acc [chains, n_vars, ldv] fp32: in kept sweeps acc[c, i, x] = acc[c, i, x] + fp32(q(x) / C(V - 1)) (float64 quotient, fp32 sum;
+ *   the first kept sweep stores the term); only columns < V are written.  samples (or NULL) [chains, n_keep, n_vars] int32: the
+ *   state after each kept sweep.  max_k: the caller's bound on k (MLBP_ERR_UNSUPPORTED above MLBP_GIBBS_MAX_K, or when
+ *   E * MLBP_GIBBS_THREADS * (4 | 8 bytes) does not fit a CTA's shared memory).  A sentence whose pair list repeats a pair or
+ *   names a variable outside [0, k) gets NaN accumulator rows.  MLBP_ERR_INVALID, nothing launched: a null pointer other than
+ *   samples, V < 1, ldv < V, ldv % 8 != 0, U / planes / acc not 16-byte aligned, chains < 1, n_keep < 1, burn_in < 0.
+ *   n_sent = 0 launches nothing.  Deterministic.                                                                                */
+#define MLBP_GIBBS_THREADS  256
+#define MLBP_GIBBS_MAX_K     64
+int mlbp_gibbs_sample(int n_sent, int max_k, int n_vars, const int32_t *var_off, const int32_t *pair_off, const int32_t *pair_v0,
+                      const int32_t *pair_v1, const int32_t *pair_gap1, const int32_t *sent_id, const float *U, const void *planes,
+                      int64_t plane_stride, int ldv, int V, int scale_exp, const double *colsums, int chains, int burn_in,
+                      int n_keep, uint64_t seed, float range_log2, float *acc, int32_t *samples, void *stream);
+/* K12 reduce.  Per variable i, m(x) = (sum over c ascending of double(acc[c, i, x])) / (chains * n_keep) in float64:
+ *   marginals[i, x] = fp32(m(x)) for x < V ([n_vars, ldv]); label_prob[i, c] = acc[c, i, label] / n_keep (float64 [n_vars, chains]);
+ *   logp_var = log m(label) (-99.99 if 0), top1 = argmax m (first index on ties), rank = #{x : m(x) > m(label)} (K5's definitions).
+ *   MLBP_ERR_INVALID, nothing launched: a null pointer, V < 1, ldv < V, ldv % 8 != 0, misaligned acc / marginals, chains < 1,
+ *   n_keep < 1.  n_vars = 0 is a no-op.                                                                                          */
+int mlbp_gibbs_reduce(int n_vars, int chains, int n_keep, const float *acc, int ldv, int V, const int32_t *var_label,
+                      float *marginals, double *label_prob, double *logp_var, int32_t *top1, int32_t *rank, void *stream);
 /* rows[0] = 1.0f (the constant-one row the kernels read for a message that is still uniform), rows[1 + t] = the message of a
  *   pairwise factor of message table t (MLBP_TABLE_T .. T1T) that is fed the uniform initial message (LBP.py:211-216 +
  *   :509 / :518): the row / column sums of the table, mean-one scaled.  rows: [MLBP_D_CONST_ROWS, ldv] fp32; the engine

@@ -37,6 +37,8 @@ _SIGNATURES = {
     'mlbp_joint_logp': 'ii' + 'ppp' + 'pppp' + 'pppp' + 'ppppii' + 'ppi' + 'pi' + 'pp' + 'p',
     'mlbp_factor_to_var_maxprod': 'ppliii' + 'ppiii' + 'pi' + 'pli' + 'p',
     'mlbp_assignment_score': 'iii' + 'pppppppp' + 'pppppppp' + 'pp' + 'ii' + 'ppp' + 'p',
+    'mlbp_gibbs_sample': 'iii' + 'pppppppp' + 'l' + 'iii' + 'p' + 'iii' + 'lf' + 'pp' + 'p',
+    'mlbp_gibbs_reduce': 'iiipiip' + 'ppppp' + 'p',
     'mlbp_plan_compile': 'ipppppp' + 'iip',
     'mlbp_plan_sizes': 'pp',
     'mlbp_plan_export': 'pp',

@@ -228,9 +228,12 @@ class Result(object):
     """Outputs of one Engine.run: tensors stay on the device until read."""
 
     def __init__(self, grad, logp, logp_var, top1, rank, beliefs, stats, messages=None, topk=None, logp_joint=None,
-                 map_score=None, label_score=None):
+                 map_score=None, label_score=None, label_prob=None, samples=None):
         self.grad, self.logp, self.logp_var, self.top1, self.rank, self.beliefs, self.stats = \
             grad, logp, logp_var, top1, rank, beliefs, stats
+        # Engine.sample: [n_vars, chains] float64, each chain's Rao-Blackwell estimate of the label's probability, and (want_samples)
+        # [chains, n_keep, n_vars] int32, the joint draws (state after each kept sweep)
+        self.label_prob, self.samples = label_prob, samples
         # want_joint: [n_sent] float64, each sentence's joint log-likelihood of its labels, the Bethe estimate at the final
         # messages (mlbp_joint_logp); -inf where a label has belief 0.  `logp` is the sum of MARGINAL log-probabilities.
         self.logp_joint = logp_joint
@@ -1011,6 +1014,98 @@ class Engine(object):
                                         _p(offsets)))
         self.launches += 1
         return text, offsets
+
+    # ------------------------------------------------------------------ Gibbs sampling (K12)
+    def unary_rows(self, corpus):
+        """K1 for every variable of `corpus` under the current theta: (U [n_vars, ld] fp32, g_unary [n_vars, 9]) device tensors"""
+        dev, ld, V, k, m, td = self.device, self.ld, self.V, self.k, self.model, self.theta_ed
+        c = lambda name: _p(corpus.dev(name, dev))
+        nv = corpus.n_vars
+        inv_sigma = torch.empty(max(nv, 1), dtype=torch.float64, device=dev)
+        g_unary = torch.empty((max(nv, 1), 9), dtype=torch.float64, device=dev)
+        U = torch.empty((max(nv, 1), ld), dtype=torch.float32, device=dev)
+        k.call('mlbp_unary_stats', nv, c('var_de'), c('var_label'), c('sp_off'), c('sp_en'), c('sp_feat'), c('sp_val'),
+               c('giv_off'), c('giv_label'), c('giv_gap1'), _p(m.pmi), _p(m.w1), _p(m.edT), _p(m.pedT), V, ld, _hp(td),
+               _p(self.edstats), _p(self.colsums), _p(inv_sigma), _p(g_unary))
+        self._timed('K1 unary_products', lambda: (3.0 * nv + len(corpus.giv_label)) * V * 4,
+                    lambda: k.call('mlbp_unary_products', nv, c('var_de'), c('sp_off'), c('sp_en'), c('sp_feat'), c('sp_val'),
+                                   c('giv_off'), c('giv_label'), c('giv_gap1'), _p(m.edT), _p(m.pedT), V, ld, _hp(td),
+                                   _p(inv_sigma), _p(self.planes), V * ld, ld, self.scale_exp, _p(self.colsums), _p(U)))
+        self.launches += 2
+        return U, g_unary
+
+    def sample(self, corpus, chains=4, burn_in=100, n_keep=100, seed=0, sent_ids=None, want_beliefs=False, want_samples=False):
+        """Gibbs sampling of each sentence's joint guesses from the model's own distribution (K12): `chains` independent chains
+        per sentence, a systematic scan over the sentence's variables, sweep 0 drawn from the unary factors alone, `burn_in`
+        sweeps discarded and `n_keep` kept.  The draws are keyed by (seed, sent_ids[s], chain, sweep, variable), so a sentence's
+        chains do not depend on the batch it is sampled in.  sent_ids: int [n_sent], default 0 .. n_sent - 1.
+        Returns a Result whose logp_var, logp, top1, rank and (want_beliefs) beliefs are the Monte Carlo estimates (the chains'
+        Rao-Blackwellised marginals averaged), with label_prob [n_vars, chains] and (want_samples) samples [chains, n_keep, n_vars];
+        grad is None.  Needs set_theta (either with_grad); reads no schedule and leaves every sum-product buffer alone."""
+        assert self.theta_ee is not None, 'set_theta first'
+        n = corpus.n_sent
+        sent_ids = np.arange(n, dtype=np.int32) if sent_ids is None else np.ascontiguousarray(sent_ids, dtype=np.int32)
+        assert sent_ids.shape == (n,), sent_ids.shape
+        # micro-batches whose accumulators [chains, n_vars, ld], U, marginals and samples fit the workspace
+        k_s = np.diff(corpus.var_off).astype(np.int64)
+        need = k_s * self.ld * 4 * (max(int(chains), 1) + 2) + (k_s * 4 * max(int(chains), 1) * max(int(n_keep), 1)
+                                                               if want_samples else 0)
+        parts, lo, used = [], 0, 0
+        for s in range(n):
+            if used + need[s] > self.workspace_bytes and s > lo:
+                parts.append((lo, s))
+                lo, used = s, 0
+            used += int(need[s])
+        parts.append((lo, n))
+        outs = [self._sample_part(corpus.slice(a, b) if (a, b) != (0, n) else corpus, sent_ids[a:b], chains, burn_in, n_keep,
+                                  seed, want_beliefs, want_samples) for a, b in parts]
+        cat = lambda xs, dim=0: None if xs[0] is None else (xs[0] if len(xs) == 1 else torch.cat(xs, dim))
+        col = lambda i, dim=0: cat([o[i] for o in outs], dim)
+        return Result(None, col(0), col(1), col(2), col(3), col(4), {'chains': chains, 'burn_in': burn_in, 'n_keep': n_keep,
+                      'micro_batches': len(parts)}, label_prob=col(5), samples=col(6, 2))
+
+    def _sample_part(self, corpus, sent_ids, chains, burn_in, n_keep, seed, want_beliefs, want_samples):
+        """K1, K12, its reduce and the per-sentence log sums of one micro-batch: (logp, logp_var, top1, rank, beliefs, label_prob,
+        samples)"""
+        dev, ld, V, k, m = self.device, self.ld, self.V, self.k, self.model
+        nv, ns = corpus.n_vars, corpus.n_sent
+        z = lambda *shape, dt=torch.float64: torch.zeros(shape, dtype=dt, device=dev)
+        if ns == 0:
+            return (z(0), z(0), z(0, dt=torch.int32), z(0, dt=torch.int32), z(0, ld, dt=torch.float32) if want_beliefs else None,
+                    z(0, max(int(chains), 1)), z(max(int(chains), 1), max(int(n_keep), 1), 0, dt=torch.int32) if want_samples else None)
+        c = lambda name: _p(corpus.dev(name, dev))
+        U, g_unary = self.unary_rows(corpus)
+        # |log2| bound of a conditional: K1's row plus every neighbour column counted as a mean-one given token (K3's range_log2)
+        deg = np.zeros(nv, dtype=np.int64)
+        first = np.repeat(corpus.var_off[:-1], np.diff(corpus.pair_off))
+        np.add.at(deg, first + corpus.pair_v0, 1)
+        np.add.at(deg, first + corpus.pair_v1, 1)
+        g_max = int(np.diff(corpus.giv_off).max())
+        range_log2 = float(2 * (g_max + int(deg.max())) * self.half_range_log2 + self.unary_range_log2)
+        sid = torch.from_numpy(np.ascontiguousarray(sent_ids, dtype=np.int32)).to(dev)
+        acc = torch.empty((max(int(chains), 1), nv, ld), dtype=torch.float32, device=dev)
+        samples = torch.empty((max(int(chains), 1), max(int(n_keep), 1), nv), dtype=torch.int32, device=dev) if want_samples else None
+        seed64 = int(seed) & 0xffffffffffffffff
+        seed64 = seed64 - (1 << 64) if seed64 >= (1 << 63) else seed64    # the uint64 key travels as an int64 argument
+        sweeps = 1 + int(burn_in) + int(n_keep)
+        n_nb = int(2 * corpus.n_pairs)
+        self._timed('K12 gibbs_sample', lambda: chains * ((sweeps * nv + (sweeps - 1) * n_nb) * V * 4.0 + int(n_keep) * nv * V * 8.0),
+                    lambda: k.call('mlbp_gibbs_sample', ns, int(np.diff(corpus.var_off).max()), nv, c('var_off'), c('pair_off'),
+                                   c('pair_v0'), c('pair_v1'), c('pair_gap1'), _p(sid), _p(U), _p(self.planes), V * ld, ld, V,
+                                   self.scale_exp, _p(self.colsums), int(chains), int(burn_in), int(n_keep), seed64, range_log2,
+                                   _p(acc), _p(samples)))
+        marg = torch.zeros((nv, ld), dtype=torch.float32, device=dev)
+        label_prob = torch.empty((nv, max(int(chains), 1)), dtype=torch.float64, device=dev)
+        logp_var = torch.empty(nv, dtype=torch.float64, device=dev)
+        top1 = torch.empty(nv, dtype=torch.int32, device=dev)
+        rank = torch.empty(nv, dtype=torch.int32, device=dev)
+        k.call('mlbp_gibbs_reduce', nv, int(chains), int(n_keep), _p(acc), ld, V, c('var_label'), _p(marg), _p(label_prob),
+               _p(logp_var), _p(top1), _p(rank))
+        grad, logp = torch.empty((ns, 9), dtype=torch.float64, device=dev), torch.empty(ns, dtype=torch.float64, device=dev)
+        k.call('mlbp_gradient_reduce', ns, c('var_off'), None, _p(g_unary), _p(z(1, 3)), None, None, c('var_label'), None, _p(m.pmi),
+               _p(m.w1), ld, _p(logp_var), _p(grad), _p(logp))
+        self.launches += 3
+        return logp, logp_var, top1, rank, marg if want_beliefs else None, label_prob, samples
 
     # ------------------------------------------------------------------ micro-batching
     def microbatches(self, corpus, sweeps, want_grad):

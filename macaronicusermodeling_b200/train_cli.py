@@ -57,6 +57,8 @@ def parse(argv=None):
     opt.add_argument('--joint_likelihood', dest='joint_likelihood', default=False, action='store_true')
     # not a reference flag: also decode each sentence's most probable joint guess (max-product BP, Engine.run max_product)
     opt.add_argument('--map_decode', dest='map_decode', default=False, action='store_true')
+    # not a reference flag: also sample every sentence's joint guesses (Gibbs, Engine.sample): N burn-in and N kept sweeps, 4 chains
+    opt.add_argument('--gibbs', dest='gibbs', type=int, default=None)
     return opt.parse_args(argv)
 
 
@@ -203,7 +205,42 @@ def merge_parts(path, parts, spans):
             os.remove(p)
 
 
-def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None, out_path=None, joint=False, map_decode=False):
+class SentenceLines(object):
+    """A one-line-per-sentence output file (.joint, .map, .gibbs): each rank writes the lines of its sentences to
+    <path>.rank<r>.part and, after a barrier, rank 0 merges the parts in file order."""
+
+    def __init__(self, path, rank, world):
+        self.path, self.rank, self.world = path, rank, world
+        self.parts = [path + '.rank%d.part' % r for r in range(world)]
+        self.f = open(self.parts[rank], 'wb')
+        self.spans, self.off = [], 0                            # (sentence, offset, length)
+
+    def write(self, i, line):
+        n = self.f.write(line.encode('utf8'))
+        self.spans.append((i, self.off, n))
+        self.off += n
+
+    def merge(self, n_sents):
+        self.f.close()
+        every = [self.spans]
+        if self.world > 1:
+            import torch.distributed as dist
+            every = [None] * self.world
+            dist.all_gather_object(every, self.spans)
+            dist.barrier()
+        if self.rank == 0:
+            where = [None] * n_sents
+            for rr, sp in enumerate(every):
+                for i, o, n in sp:
+                    where[i] = (rr, o, n)
+            merge_parts(self.path, self.parts, where)
+
+
+GIBBS_CHAINS = 4
+
+
+def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None, out_path=None, joint=False, map_decode=False,
+            gibbs=0):
     """train.py:308-338 batched and sharded over the torchrun ranks.  `units`: prediction_units(); `thetas`: domain ->
     (theta_ee, theta_ed) for the adaptation modes (else the engine's current theta is used).  The roots of every sentence are
     drawn from `rng` in unit order before the units are shared out, so a sentence gets the same roots on any number of ranks.
@@ -214,7 +251,12 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
     the file <out_path>.joint, one line  sent_id TAB joint TAB sum of marginal logp  per sentence in file order.
     `map_decode`: every unit also runs max-product inference with the same roots (no further draws from `rng`); one more result
     (tokens whose decoded word is the label, sentences decoded entirely right), and with `out_path` the file <out_path>.map, one
-    line  sent_id TAB decoded words in position order TAB map_score TAB label_score  per sentence in file order."""
+    line  sent_id TAB decoded words in position order TAB map_score TAB label_score  per sentence in file order.
+    `gibbs` = N > 0: every unit is also sampled (Engine.sample: 4 chains, N burn-in and N kept sweeps, key options.seed, the
+    sentence's line index as its id; no draws from `rng`); one more result (sum over sentences of the Monte Carlo sum of log
+    p(label), #rank == 0, largest across-chain standard error of a label probability), and with `out_path` the file
+    <out_path>.gibbs, one line  sent_id TAB Gibbs log p(label) TAB standard errors TAB BP logp_var  (per token in position order)
+    per sentence in file order."""
     import torch
     from .engine import Corpus
     from .trainer import dist_info
@@ -222,24 +264,18 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
     V = len(en_domain)
     corpora = [Corpus([sents[i] for i in idx]) for _, idx in units]
     roots = [draw_roots(c, 3, rng) for c in corpora]
-    # per unit: sum logp, #rank == 0, < 26, < 50, variables, sum joint, MAP tokens right, MAP sentences right
-    stats = np.zeros((len(units), 8))
+    # per unit: sum logp, #rank == 0, < 26, < 50, variables, sum joint, MAP tokens right, MAP sentences right, Gibbs sum logp,
+    # Gibbs #rank == 0, largest Gibbs standard error
+    stats = np.zeros((len(units), 11))
     write = bool(out_path) and not qp
     if write:
         parts = [out_path + '.rank%d.part' % r for r in range(world)]
         dparts = [out_path + '.dist.rank%d.part' % r for r in range(world)]
         wp, wd = open(parts[rank], 'wb'), open(dparts[rank], 'wb')
         spans, p_off, d_off = [], 0, 0                          # (sentence, .pred offset, length, .dist offset, length)
-    write_joint = bool(out_path) and joint
-    if write_joint:
-        jparts = [out_path + '.joint.rank%d.part' % r for r in range(world)]
-        wj = open(jparts[rank], 'wb')
-        jspans, j_off = [], 0                                   # (sentence, .joint offset, length)
-    write_map = bool(out_path) and map_decode
-    if write_map:
-        mparts = [out_path + '.map.rank%d.part' % r for r in range(world)]
-        wm = open(mparts[rank], 'wb')
-        mspans, m_off = [], 0                                   # (sentence, .map offset, length)
+    wj = SentenceLines(out_path + '.joint', rank, world) if (out_path and joint) else None
+    wm = SentenceLines(out_path + '.map', rank, world) if (out_path and map_decode) else None
+    wg = SentenceLines(out_path + '.gibbs', rank, world) if (out_path and gibbs) else None
     pinned = [None]
     cur = object()
     for u in range(rank, len(units), world):
@@ -255,27 +291,36 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
         if joint:
             lj = r.logp_joint.cpu().numpy()
             stats[u, 5] = float(lj.sum())
-        if write_joint:
+        if wj:
             lm = r.logp.cpu().numpy()
             for si, i in enumerate(idx):
                 nodes = sorted(raw[i]['current_sent'], key=lambda n: int(n['position']))
-                j_len = wj.write(('%s\t%r\t%r\n' % (nodes[0]['sent_id'], float(lj[si]), float(lm[si]))).encode('utf8'))
-                jspans.append((i, j_off, j_len))
-                j_off += j_len
+                wj.write(i, '%s\t%r\t%r\n' % (nodes[0]['sent_id'], float(lj[si]), float(lm[si])))
         if map_decode:
             rm = engine.run(corpus, roots[u], 3, want_grad=False, want_marg=True, max_product=True)
             dec, lab = rm.top1.cpu().numpy(), corpus.var_label
             ok = dec == lab
             stats[u, 6] = int(ok.sum())
             stats[u, 7] = sum(1 for si in range(len(idx)) if ok[corpus.var_off[si]:corpus.var_off[si + 1]].all())
-            if write_map:
+            if wm:
                 ms, ls = rm.map_score.cpu().numpy(), rm.label_score.cpu().numpy()
                 for si, i in enumerate(idx):
                     nodes = sorted(raw[i]['current_sent'], key=lambda n: int(n['position']))
                     words = ' '.join(en_domain[int(e)] for e in dec[corpus.var_off[si]:corpus.var_off[si + 1]])
-                    m_len = wm.write(('%s\t%s\t%r\t%r\n' % (nodes[0]['sent_id'], words, float(ms[si]), float(ls[si]))).encode('utf8'))
-                    mspans.append((i, m_off, m_len))
-                    m_off += m_len
+                    wm.write(i, '%s\t%s\t%r\t%r\n' % (nodes[0]['sent_id'], words, float(ms[si]), float(ls[si])))
+        if gibbs:
+            rg = engine.sample(corpus, chains=GIBBS_CHAINS, burn_in=gibbs, n_keep=gibbs, seed=options.seed,
+                               sent_ids=np.asarray(idx, dtype=np.int32))
+            glv, grk = rg.logp_var.cpu().numpy(), rg.rank.cpu().numpy()
+            se = rg.label_prob.cpu().numpy().std(axis=1, ddof=1) / np.sqrt(GIBBS_CHAINS)
+            stats[u, 8:11] = (float(rg.logp.sum().item()), int((grk == 0).sum()), float(se.max()))
+            if wg:
+                blv = r.logp_var.cpu().numpy()
+                for si, i in enumerate(idx):
+                    nodes = sorted(raw[i]['current_sent'], key=lambda n: int(n['position']))
+                    lo, hi = int(corpus.var_off[si]), int(corpus.var_off[si + 1])
+                    cols = [' '.join('%r' % float(v) for v in a[lo:hi]) for a in (glv, se, blv)]
+                    wg.write(i, '\t'.join([str(nodes[0]['sent_id'])] + cols) + '\n')
         if not write:
             continue
         text, toff = dist_text(engine, r.beliefs, pinned)
@@ -333,34 +378,11 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
                     where[i] = (rr, po, pl, do, dl)
             merge_parts(out_path, parts, [(w[0], w[1], w[2]) for w in where])
             merge_parts(out_path + '.dist', dparts, [(w[0], w[3], w[4]) for w in where])
-    if write_joint:
-        wj.close()
-        every = [jspans]
-        if world > 1:
-            every = [None] * world
-            dist.all_gather_object(every, jspans)
-            dist.barrier()
-        if rank == 0:
-            where = [None] * len(sents)
-            for rr, sp in enumerate(every):
-                for i, jo, jl in sp:
-                    where[i] = (rr, jo, jl)
-            merge_parts(out_path + '.joint', jparts, where)
-    if write_map:
-        wm.close()
-        every = [mspans]
-        if world > 1:
-            every = [None] * world
-            dist.all_gather_object(every, mspans)
-            dist.barrier()
-        if rank == 0:
-            where = [None] * len(sents)
-            for rr, sp in enumerate(every):
-                for i, mo, ml in sp:
-                    where[i] = (rr, mo, ml)
-            merge_parts(out_path + '.map', mparts, where)
+    for w in (wj, wm, wg):
+        if w:
+            w.merge(len(sents))
     sums = []
-    for col in (0, 5):
+    for col in (0, 5, 8):
         total, k = 0.0, 0
         while k < len(units):                                   # one partial sum per domain, as the single-process loop
             part, d = 0.0, units[k][0]
@@ -375,6 +397,8 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
         out += (sums[1],)
     if map_decode:
         out += (tuple(int(x) for x in stats[:, 6:8].sum(axis=0)),)
+    if gibbs:
+        out += ((sums[2], int(stats[:, 9].sum()), float(stats[:, 10].max()) if len(units) else 0.0),)
     return out
 
 
@@ -383,6 +407,14 @@ def print_map(prefix, counts, n_tokens, n_sents):
     print(prefix + 'prediction MAP token accuracy:', '%0.2f' % (float(100 * counts[0]) / float(max(n_tokens, 1))), 'total:', n_tokens)
     print(prefix + 'prediction MAP sentence accuracy:', '%0.2f' % (float(100 * counts[1]) / float(max(n_sents, 1))), 'total:',
           n_sents)
+
+
+def print_gibbs(prefix, res, n_lines, n_tokens):
+    """the three --gibbs lines: the Monte Carlo counterpart of `prediction probs:` and of `Prec at 0:`, and the largest
+    across-chain standard error of a label probability"""
+    print(prefix + 'prediction Gibbs probs:', res[0] / float(n_lines))
+    print(prefix + 'prediction Gibbs Prec at 0:', '%0.2f' % (float(100 * res[1]) / float(max(n_tokens, 1))), 'total:', n_tokens)
+    print(prefix + 'prediction Gibbs max standard error:', res[2])
 
 
 def main(argv=None):
@@ -398,6 +430,9 @@ def main(argv=None):
     if options.map_decode and (options.use_approx_inference or options.use_approx_beliefs):
         sys.stderr.write('--map_decode decodes with exact max-product inference: it does not combine with --use_approx_inference '
                          'or --use_approx_beliefs\n')
+        return 1
+    if options.gibbs is not None and options.gibbs < 1:
+        sys.stderr.write('--gibbs N needs N >= 1 (burn-in and kept sweeps per chain)\n')
         return 1
     adapt = options.user_adapt or options.experience_adapt
     import os
@@ -508,7 +543,8 @@ def main(argv=None):
                 engine.set_theta(tr.theta_ee, tr.theta_ed, with_grad=True)
                 tune_sents = lower(tune_lines, options, en2id, de2id)
                 res = predict(engine, prediction_units(len(tune_sents)), tune_sents, [json.loads(l) for l in tune_lines],
-                              en_domain, options, rng, True, joint=options.joint_likelihood, map_decode=options.map_decode)
+                              en_domain, options, rng, True, joint=options.joint_likelihood, map_decode=options.map_decode,
+                              gibbs=options.gibbs or 0)
                 lp, (p0, p25, p50, tot) = res[:2]
                 if rank == 0:
                     print('\ntune prediction probs:', lp / float(len(tune_lines)))
@@ -517,7 +553,9 @@ def main(argv=None):
                     if options.joint_likelihood:
                         print('tune prediction joint log-likelihood:', res[2] / float(len(tune_lines)))
                     if options.map_decode:
-                        print_map('tune ', res[-1], tot, len(tune_sents))
+                        print_map('tune ', res[2 + bool(options.joint_likelihood)], tot, len(tune_sents))
+                    if options.gibbs:
+                        print_gibbs('tune ', res[-1], len(tune_lines), tot)
         print('\ntheta final:', tr.theta_ee, tr.theta_ed)
         if rank == 0 and options.save_params_file:
             save_params(codecs.open(options.save_params_file, 'w', 'utf8'), tr.theta_ee.reshape(1, -1), tr.theta_ed.reshape(1, -1),
@@ -535,7 +573,8 @@ def main(argv=None):
         engine.set_theta(theta_ee.reshape(-1), theta_ed.reshape(-1), with_grad=True)
         thetas, units = None, prediction_units(len(all_sents))
     res = predict(engine, units, all_sents, raw, en_domain, options, rng, options.quick_predict, thetas,
-                  options.save_predictions_file, joint=options.joint_likelihood, map_decode=options.map_decode)
+                  options.save_predictions_file, joint=options.joint_likelihood, map_decode=options.map_decode,
+                  gibbs=options.gibbs or 0)
     lp, (p0, p25, p50, tot) = res[:2]
     if rank == 0:
         print('\nprediction probs:', lp / float(len(train_lines)))
@@ -544,7 +583,9 @@ def main(argv=None):
         if options.joint_likelihood:
             print('prediction joint log-likelihood:', res[2] / float(len(train_lines)))
         if options.map_decode:
-            print_map('', res[-1], tot, len(all_sents))
+            print_map('', res[2 + bool(options.joint_likelihood)], tot, len(all_sents))
+        if options.gibbs:
+            print_gibbs('', res[-1], len(train_lines), tot)
     if torch.cuda.is_available():
         torch.cuda.synchronize()
     return 0

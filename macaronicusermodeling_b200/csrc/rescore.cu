@@ -62,7 +62,7 @@ rescore_kernel(const int32_t *__restrict__ flagged, const int32_t *__restrict__ 
     __shared__ int s_bits[RS_MAX_CAND];
     __shared__ double s_score[RS_MAX_CAND];
     __shared__ double s_dot[RS_MAX_CAND];
-    __shared__ int s_nc;
+    __shared__ int s_nc, s_ref;
     const int total = *n_flagged;
     for (int it = blockIdx.x; it < total; it += gridDim.x) {
         const int g = flagged[it];
@@ -129,7 +129,17 @@ rescore_kernel(const int32_t *__restrict__ flagged, const int32_t *__restrict__ 
             if (threadIdx.x == 0) atomicAdd(&counters[1], 1);
             continue;
         }
-        if (threadIdx.x < nc) s_score[threadIdx.x] = (double)__ldg(urow + s_cand[threadIdx.x]) / (double)__ldg(urow + s_cand[0]);
+        // scores are ratios to one reference candidate.  The arg-max does not depend on the label, so with bit 0 the reference
+        // is the bit-0 candidate of smallest index (a label whose product is 0 must not stop the arg-max re-score); else the label
+        if (threadIdx.x == 0) {
+            int k = 0;
+            for (int c = 1; c < nc; ++c)
+                if ((s_bits[c] & 1) && (!(s_bits[k] & 1) || s_cand[c] < s_cand[k])) k = c;
+            s_ref = k;
+        }
+        __syncthreads();
+        const int ref = s_ref;
+        if (threadIdx.x < nc) s_score[threadIdx.x] = (double)__ldg(urow + s_cand[threadIdx.x]) / (double)__ldg(urow + s_cand[ref]);
         __syncthreads();
         // ---- exact last hop, one incoming message at a time
         bool bad = false;
@@ -184,13 +194,13 @@ rescore_kernel(const int32_t *__restrict__ flagged, const int32_t *__restrict__ 
                 }
             }
             __syncthreads();
-            const double d0 = s_dot[0];
+            const double d0 = s_dot[ref];
             if (!(d0 > 0.0) || !isfinite(d0)) bad = true;          // block-uniform
             if (!bad && threadIdx.x < nc) s_score[threadIdx.x] *= s_dot[threadIdx.x] / d0;
             __syncthreads();
         }
         if (threadIdx.x == 0) {
-            bool ok = !bad;
+            bool ok = !bad && (!(flag & 2) || s_score[0] > 0.0);  // a rank needs a positive label product
             for (int c = 0; c < nc; ++c) ok = ok && isfinite(s_score[c]);
             if (!ok) {
                 atomicAdd(&counters[2], 1);                        // degenerate products: keep K5's answer

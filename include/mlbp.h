@@ -402,6 +402,38 @@ int mlbp_gibbs_sample(int n_sent, int max_k, int n_vars, const int32_t *var_off,
  *   n_keep < 1.  n_vars = 0 is a no-op.                                                                                          */
 int mlbp_gibbs_reduce(int n_vars, int chains, int n_keep, const float *acc, int ldv, int V, const int32_t *var_label,
                       float *marginals, double *label_prob, double *logp_var, int32_t *top1, int32_t *rank, void *stream);
+/* K13. Pseudo-likelihood of each sentence's labels (not in the reference): for every variable i of a sentence (variables
+ *   [var_off[s], var_off[s + 1]), k of them, pairwise factors [pair_off[s], ..) with local pair_v0 / pair_v1 as in
+ *   mlbp_gibbs_sample) the exact conditional of its label y_i = var_label[i] given the other variables' labels,
+ *     p(y_i | y_-i) = q_i(y_i) / Z_i,   Z_i = sum_{x < V} q_i(x),
+ *   with q_i formed exactly as K12 forms a conditional (same planes, factor f, order and product rounding; fp64 products when
+ *   range_log2 is outside [0, 100)) with the labels as the other variables' words, and Z_i summed in K12's block order
+ *   (E, the thread sums, the Kogge-Stone scan and the warp totals of mlbp_gibbs_sample: Z_i is K12's C(V - 1)).
+ *   One CTA of MLBP_GIBBS_THREADS threads per variable.  Outputs per variable:
+ *     logp_var[i] = log(q_i(y_i) / Z_i) (-99.99 where q_i(y_i) = 0); top1[i] = argmax q_i (first index on ties);
+ *     rank[i] = #{x : q_i(x) > q_i(y_i)}; beliefs (or NULL) [n_vars, ldv] fp32: q_i / Z_i at columns < V (nothing else written).
+ *   grad (or NULL) [n_vars, 9], laid out like g_unary: the exact gradient of log p(y_i | y_-i),  phi(y_i) - E_p[phi]  summed over
+ *     the en_de factor (edT / pedT row var_de[i], none where var_de < 0; sparse entries (e, f, val): val ([y_i == e] - p(e))),
+ *     every given token j (pmi / pmi_w1 column giv_label[j], pmi_w1 where giv_gap1) and every pairwise factor touching i
+ *     (pmi / pmi_w1 at the factor's orientation, pmi_w1 where pair_gap1).  The observed values are read from the fp32 planes
+ *     pmi, pmi_w1 [V, ldf], edT, pedT [Vd, ldf]; E_p[pmi(., y)] = sum_x p(x) G_y(x) / T_y(x) with T_y the table row of the product
+ *     and G_y the same row of the gradient planes 8..19 (a column with p(x) = 0 contributes 0), fp32 per thread, float64 across
+ *     the block in a fixed order.  The bias components are exactly 0.  Needs planes built with_grad_planes.  Deterministic.
+ *   A variable whose sentence's pair list cannot be read (as in K12), or whose sentence names a label or given word outside
+ *   [0, V), gets logp_var = NaN, grad = NaN, beliefs = NaN, top1 = -1, rank = INT_MAX; nothing is read out of bounds.
+ *   MLBP_ERR_UNSUPPORTED: max_k > MLBP_PL_MAX_K (Corpus.MAX_PREDICTED), or E * MLBP_GIBBS_THREADS * (4 | 8 bytes) does not fit a
+ *   CTA's shared memory.  MLBP_ERR_INVALID, nothing launched: a null pointer (var_de, the sparse lists and the fp32 planes may
+ *   be NULL without grad), V < 1, ldv < V, ldv % 8 != 0, plane_stride < V ldv, with grad ldf < V or ldf % 8 != 0, U / planes /
+ *   beliefs / edT / pedT not 16-byte aligned, max_k < 1.  n_sent = 0 or n_vars = 0 launches nothing.                       */
+#define MLBP_PL_MAX_K        49
+int mlbp_pseudo_likelihood(int n_sent, int max_k, int n_vars, const int32_t *var_off, const int32_t *pair_off,
+                           const int32_t *pair_v0, const int32_t *pair_v1, const int32_t *pair_gap1, const int32_t *var_label,
+                           const int32_t *var_de, const int32_t *sp_off, const int32_t *sp_en, const int32_t *sp_feat,
+                           const float *sp_val, const int32_t *giv_off, const int32_t *giv_label, const int32_t *giv_gap1,
+                           const float *U, const void *planes, int64_t plane_stride, int ldv, int V, int scale_exp,
+                           const double *colsums, const float *pmi, const float *pmi_w1, const float *edT, const float *pedT,
+                           int ldf, float range_log2, double *logp_var, int32_t *top1, int32_t *rank, double *grad,
+                           float *beliefs, void *stream);
 /* rows[0] = 1.0f (the constant-one row the kernels read for a message that is still uniform), rows[1 + t] = the message of a
  *   pairwise factor of message table t (MLBP_TABLE_T .. T1T) that is fed the uniform initial message (LBP.py:211-216 +
  *   :509 / :518): the row / column sums of the table, mean-one scaled.  rows: [MLBP_D_CONST_ROWS, ldv] fp32; the engine

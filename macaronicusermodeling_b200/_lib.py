@@ -39,6 +39,7 @@ _SIGNATURES = {
     'mlbp_assignment_score': 'iii' + 'pppppppp' + 'pppppppp' + 'pp' + 'ii' + 'ppp' + 'p',
     'mlbp_gibbs_sample': 'iii' + 'pppppppp' + 'l' + 'iii' + 'p' + 'iii' + 'lf' + 'pp' + 'p',
     'mlbp_gibbs_reduce': 'iiipiip' + 'ppppp' + 'p',
+    'mlbp_pseudo_likelihood': 'iii' + 'ppppp' + 'pppppp' + 'ppp' + 'pp' + 'l' + 'iii' + 'p' + 'pppp' + 'i' + 'f' + 'ppppp' + 'p',
     'mlbp_plan_compile': 'ipppppp' + 'iip',
     'mlbp_plan_sizes': 'pp',
     'mlbp_plan_export': 'pp',

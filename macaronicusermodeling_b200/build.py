@@ -10,7 +10,7 @@ LIB = os.path.join(HERE, 'libmlbp.so')
 STAMP = os.path.join(HERE, 'libmlbp.so.stamp')
 SOURCES = ['api.cu', 'tables.cu', 'unary.cu', 'messages.cu', 'gemm_simt.cu', 'gemm_tcgen05.cu', 'gradient.cu',
            'dense.cu', 'rescore.cu', 'spikes.cu', 'topk.cu', 'format.cu', 'parse.cu', 'joint.cu', 'maxprod.cu',
-           'gibbs.cu', 'plan.cpp']
+           'gibbs.cu', 'pseudo.cu', 'plan.cpp']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17', '--use_fast_math=false',
               '-Xcompiler', '-fPIC', '-Xcompiler', '-fvisibility=default']
 

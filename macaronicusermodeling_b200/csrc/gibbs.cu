@@ -5,14 +5,11 @@
 // words act like given tokens), takes the float64 running sum of q in a fixed block-wide order, draws x_i with a counter-based
 // Philox uniform and, in kept sweeps, adds q_i / sum to the chain's Rao-Blackwell row.  Everything is ordered so that a NumPy
 // emulation (tests/gibbs_oracle.py) reproduces every q, every sum and every draw bit for bit.
-#include "common.cuh"
+#include "conditional.cuh"
 
 #include <limits.h>
 
 namespace mlbp {
-
-constexpr int GT = MLBP_GIBBS_THREADS;
-constexpr int GW = GT / 32;
 
 // Philox4x32-10 (Salmon et al., SC'11; the constants of Random123), counter c, key (k0, k1)
 __host__ __device__ __forceinline__ void philox4x32_10(uint32_t c[4], uint32_t k0, uint32_t k1) {
@@ -25,23 +22,6 @@ __host__ __device__ __forceinline__ void philox4x32_10(uint32_t c[4], uint32_t k
         c[3] = lo0;
         k0 += 0x9E3779B9u;
         k1 += 0xBB67AE85u;
-    }
-}
-
-__device__ __forceinline__ double to_d(float v) { return (double)v; }
-__device__ __forceinline__ double to_d(double v) { return v; }
-// one factor of the conditional: q * ((hi + lo) * f), every operation rounded on its own (no contraction)
-__device__ __forceinline__ float mul_factor(float q, float t, float f) { return __fmul_rn(q, __fmul_rn(t, f)); }
-__device__ __forceinline__ double mul_factor(double q, float t, float f) { return __dmul_rn(q, __dmul_rn((double)t, (double)f)); }
-
-__device__ __forceinline__ void halves8(const __half *p, float *out) {
-    const uint4 w = *reinterpret_cast<const uint4 *>(p);
-    const __half2 *h = reinterpret_cast<const __half2 *>(&w);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const float2 f = __half22float2(h[j]);
-        out[2 * j] = f.x;
-        out[2 * j + 1] = f.y;
     }
 }
 
@@ -71,27 +51,7 @@ gibbs_kernel(int max_k, const int32_t *__restrict__ var_off, const int32_t *__re
     const int p0 = pair_off[s], n_p = pair_off[s + 1] - p0;
     const int e_beg = tid * E;
     if (k < 1 || k > max_k || v0 < 0 || v0 + k > n_vars) return;     // outside the caller's stated bounds: nothing to own
-    if (tid == 0) {
-        // per variable, the factors that touch it in pair-list order: neighbour | (1 if the variable is dim 1) << 6 | gap1 << 7
-        int bad = n_p < 0 || 2 * n_p > k * (k - 1);
-        for (int i = 0; i <= k; ++i) nb_off[i] = 0;
-        for (int p = 0; p < n_p && !bad; ++p) {
-            const int a = pair_v0[p0 + p], b = pair_v1[p0 + p];
-            if (a < 0 || a >= k || b < 0 || b >= k || a == b) bad = 1;
-            else ++nb_off[a + 1], ++nb_off[b + 1];
-        }
-        for (int i = 0; i < k && !bad; ++i) {
-            bad = nb_off[i + 1] > k - 1;
-            nb_off[i + 1] += nb_off[i];
-            x[i] = nb_off[i];                                          // fill cursor
-        }
-        for (int p = 0; p < n_p && !bad; ++p) {
-            const int a = pair_v0[p0 + p], b = pair_v1[p0 + p], g = pair_gap1[p0 + p] ? 1 : 0;
-            nb[x[a]++] = (uint16_t)(b | (g << 7));
-            nb[x[b]++] = (uint16_t)(a | (1 << 6) | (g << 7));
-        }
-        s_bad = bad;
-    }
+    if (tid == 0) s_bad = build_neighbours(k, p0, n_p, pair_v0, pair_v1, pair_gap1, nb_off, x, nb);   // x: fill cursor
     __syncthreads();
     if (s_bad) {                                                       // a pair list the sampler cannot read: NaN rows
         for (int i = 0; i < k; ++i)
@@ -106,14 +66,7 @@ gibbs_kernel(int max_k, const int32_t *__restrict__ var_off, const int32_t *__re
             const int deg = sw == 0 ? 0 : nb_off[i + 1] - nb_off[i];    // sweep 0 draws from U_i alone
             if (tid < deg) {
                 const int ent = nb[nb_off[i] + tid];
-                const int j = ent & 63, dim1 = (ent >> 6) & 1, g = (ent >> 7) & 1;
-                const int y = x[j];
-                // dim 0: T[x, y] is row y of TT / T1T (planes 2 / 6) with the column sums; dim 1: T[y, x] is row y of T / T1
-                // (planes 0 / 4) with the row sums (colsums rows 5 / 6)
-                const int plane = dim1 ? (g ? 4 : 0) : (g ? 6 : 2);
-                const int sum = dim1 ? (g ? 6 : 5) : (g ? 1 : 0);
-                row_off[tid] = (int64_t)plane * ps + (int64_t)y * ldv;
-                row_f[tid] = (float)(unscale * (double)V / colsums[(size_t)sum * V + y]);
+                factor_row(ent, x, ps, ldv, V, unscale, colsums, row_off[tid], row_f[tid]);
             }
             if (tid == 0) {
                 s_hit = INT_MAX;
@@ -126,35 +79,7 @@ gibbs_kernel(int max_k, const int32_t *__restrict__ var_off, const int32_t *__re
             for (int j0 = 0; j0 < E; j0 += 8) {
                 const int e0 = e_beg + j0;
                 Q q[8];
-                if (e0 < V) {
-                    const float4 ua = *reinterpret_cast<const float4 *>(urow + e0);
-                    const float4 ub = *reinterpret_cast<const float4 *>(urow + e0 + 4);
-                    q[0] = ua.x; q[1] = ua.y; q[2] = ua.z; q[3] = ua.w;
-                    q[4] = ub.x; q[5] = ub.y; q[6] = ub.z; q[7] = ub.w;
-                    int m = 0;
-                    for (; m + 4 <= deg; m += 4) {                     // 8 independent 16-byte row loads in flight
-                        float h[4][8], l[4][8];
-#pragma unroll
-                        for (int r = 0; r < 4; ++r) {
-                            halves8(planes + row_off[m + r] + e0, h[r]);
-                            halves8(planes + row_off[m + r] + ps + e0, l[r]);
-                        }
-#pragma unroll
-                        for (int r = 0; r < 4; ++r) {
-                            const float f = row_f[m + r];
-#pragma unroll
-                            for (int jj = 0; jj < 8; ++jj) q[jj] = mul_factor(q[jj], __fadd_rn(h[r][jj], l[r][jj]), f);
-                        }
-                    }
-                    for (; m < deg; ++m) {
-                        float h[8], l[8];
-                        halves8(planes + row_off[m] + e0, h);
-                        halves8(planes + row_off[m] + ps + e0, l);
-                        const float f = row_f[m];
-#pragma unroll
-                        for (int jj = 0; jj < 8; ++jj) q[jj] = mul_factor(q[jj], __fadd_rn(h[jj], l[jj]), f);
-                    }
-                }
+                if (e0 < V) conditional8(q, urow, e0, deg, planes, row_off, row_f, ps);
 #pragma unroll
                 for (int jj = 0; jj < 8; ++jj) {
                     const Q v = (e0 + jj < V) ? q[jj] : Q(0);
@@ -162,20 +87,7 @@ gibbs_kernel(int max_k, const int32_t *__restrict__ var_off, const int32_t *__re
                     t_sum = __dadd_rn(t_sum, to_d(v));
                 }
             }
-            // block exclusive scan of the thread sums: Kogge-Stone inside a warp, the warp totals added in warp order
-            double v = t_sum;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const double y = __shfl_up_sync(0xffffffffu, v, d);
-                if (lane >= d) v = __dadd_rn(v, y);
-            }
-            double ex = __shfl_up_sync(0xffffffffu, v, 1);
-            if (lane == 0) ex = 0.0;
-            if (lane == 31) warp_tot[warp] = v;
-            __syncthreads();
-            double o = 0.0;
-            for (int w = 0; w < warp; ++w) o = __dadd_rn(o, warp_tot[w]);
-            const double base = __dadd_rn(o, ex);                      // C(e) = base + (running sum of this thread up to e)
+            const double base = scan_base(t_sum, warp_tot, lane, warp);   // C(e) = base + (running sum of this thread up to e)
             if (e_beg <= V - 1 && V - 1 < e_beg + E) s_tot = __dadd_rn(base, t_sum);
             __syncthreads();
             const double tot = s_tot;                                  // C(V - 1)

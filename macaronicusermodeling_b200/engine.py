@@ -1034,6 +1034,16 @@ class Engine(object):
         self.launches += 2
         return U, g_unary
 
+    def _conditional_range_log2(self, corpus):
+        """|log2| bound of a full conditional (K12, K13): K1's row plus every neighbour column counted as a mean-one given token
+        (K3's range_log2)"""
+        deg = np.zeros(corpus.n_vars, dtype=np.int64)
+        first = np.repeat(corpus.var_off[:-1], np.diff(corpus.pair_off))
+        np.add.at(deg, first + corpus.pair_v0, 1)
+        np.add.at(deg, first + corpus.pair_v1, 1)
+        g_max = int(np.diff(corpus.giv_off).max())
+        return float(2 * (g_max + int(deg.max())) * self.half_range_log2 + self.unary_range_log2)
+
     def sample(self, corpus, chains=4, burn_in=100, n_keep=100, seed=0, sent_ids=None, want_beliefs=False, want_samples=False):
         """Gibbs sampling of each sentence's joint guesses from the model's own distribution (K12): `chains` independent chains
         per sentence, a systematic scan over the sentence's variables, sweep 0 drawn from the unary factors alone, `burn_in`
@@ -1075,13 +1085,7 @@ class Engine(object):
                     z(0, max(int(chains), 1)), z(max(int(chains), 1), max(int(n_keep), 1), 0, dt=torch.int32) if want_samples else None)
         c = lambda name: _p(corpus.dev(name, dev))
         U, g_unary = self.unary_rows(corpus)
-        # |log2| bound of a conditional: K1's row plus every neighbour column counted as a mean-one given token (K3's range_log2)
-        deg = np.zeros(nv, dtype=np.int64)
-        first = np.repeat(corpus.var_off[:-1], np.diff(corpus.pair_off))
-        np.add.at(deg, first + corpus.pair_v0, 1)
-        np.add.at(deg, first + corpus.pair_v1, 1)
-        g_max = int(np.diff(corpus.giv_off).max())
-        range_log2 = float(2 * (g_max + int(deg.max())) * self.half_range_log2 + self.unary_range_log2)
+        range_log2 = self._conditional_range_log2(corpus)
         sid = torch.from_numpy(np.ascontiguousarray(sent_ids, dtype=np.int32)).to(dev)
         acc = torch.empty((max(int(chains), 1), nv, ld), dtype=torch.float32, device=dev)
         samples = torch.empty((max(int(chains), 1), max(int(n_keep), 1), nv), dtype=torch.int32, device=dev) if want_samples else None
@@ -1106,6 +1110,82 @@ class Engine(object):
                _p(m.w1), ld, _p(logp_var), _p(grad), _p(logp))
         self.launches += 3
         return logp, logp_var, top1, rank, marg if want_beliefs else None, label_prob, samples
+
+    # ------------------------------------------------------------------ pseudo-likelihood (K13)
+    def pseudo_likelihood(self, corpus, want_grad=True, want_beliefs=False, want_topk=0, reduce_into=None):
+        """Besag's pseudo-likelihood of each sentence's labels (K13): for every variable the exact conditional
+        p(y_i | y_-i) of its label given the labels of the other variables of its sentence, under the model BP approximates.
+        Returns a Result: logp_var [n_vars] = log p(y_i | y_-i), logp [n_sent] = their sum per sentence (the PL), top1 / rank
+        of each conditional (precision_counts counts the conditional arg-maxes), grad [n_sent, 9] = the exact gradient of
+        the PL (want_grad; None otherwise), beliefs [n_vars, ld] = the normalised conditionals (want_beliefs) and topk
+        (want_topk = K, as in run).  reduce_into: 16 float64 this call's sums are added to (as run's).  Needs set_theta, with
+        with_grad=True for want_grad.  Reads no schedule, no A / D row, no flag word and no constant row: sum-product results
+        are the same around a call.  ValueError (before any launch) for a label or given word outside [0, V)."""
+        assert self.theta_ee is not None, 'set_theta first'
+        if want_grad and not self.with_grad_planes:
+            raise ValueError('the pseudo-likelihood gradient reads the gradient planes: set_theta(..., with_grad=True)')
+        for name in ('var_label', 'giv_label'):
+            a = getattr(corpus, name)
+            if len(a) and (int(a.min()) < 0 or int(a.max()) >= self.V):
+                raise ValueError('%s outside [0, V = %d): the conditional of a word the tables do not have' % (name, self.V))
+        n = corpus.n_sent
+        # micro-batches whose U rows and (want_beliefs / want_topk) conditionals fit the workspace
+        k_s = np.diff(corpus.var_off).astype(np.int64)
+        need = k_s * self.ld * 4 * (2 if (want_beliefs or want_topk) else 1)
+        parts, lo, used = [], 0, 0
+        for s in range(n):
+            if used + need[s] > self.workspace_bytes and s > lo:
+                parts.append((lo, s))
+                lo, used = s, 0
+            used += int(need[s])
+        parts.append((lo, n))
+        outs = [self._pl_part(corpus.slice(a, b) if (a, b) != (0, n) else corpus, want_grad, want_beliefs or want_topk,
+                              reduce_into) for a, b in parts]
+        cat = lambda xs: None if xs[0] is None else (xs[0] if len(xs) == 1 else torch.cat(xs))
+        col = lambda i: cat([o[i] for o in outs])
+        beliefs = col(5)
+        topk = self.topk_rows(beliefs, min(int(want_topk), self.V)) if want_topk else None
+        return Result(col(0) if want_grad else None, col(1), col(2), col(3), col(4), beliefs if want_beliefs else None,
+                      {'micro_batches': len(parts)}, topk=topk)
+
+    def _pl_part(self, corpus, want_grad, want_rows, reduce_into):
+        """K1, K13, the per-sentence sums and (reduce_into) the batch sums of one micro-batch:
+        (grad, logp, logp_var, top1, rank, beliefs)"""
+        dev, ld, V, k, m = self.device, self.ld, self.V, self.k, self.model
+        nv, ns = corpus.n_vars, corpus.n_sent
+        if ns == 0:
+            z = lambda *shape, dt=torch.float64: torch.zeros(shape, dtype=dt, device=dev)
+            return (z(0, 9), z(0), z(0), z(0, dt=torch.int32), z(0, dt=torch.int32), z(0, ld, dt=torch.float32) if want_rows else None)
+        c = lambda name: _p(corpus.dev(name, dev))
+        U, _ = self.unary_rows(corpus)
+        logp_var = torch.empty(nv, dtype=torch.float64, device=dev)
+        top1 = torch.empty(nv, dtype=torch.int32, device=dev)
+        rank = torch.empty(nv, dtype=torch.int32, device=dev)
+        g = torch.empty((nv, 9), dtype=torch.float64, device=dev) if want_grad else torch.zeros((nv, 9), dtype=torch.float64, device=dev)
+        rows = torch.zeros((nv, ld), dtype=torch.float32, device=dev) if want_rows else None
+        n_nb, n_giv = 2 * corpus.n_pairs, len(corpus.giv_label)
+        n_gap1 = 2 * int(corpus.pair_gap1.sum()) + int(corpus.giv_gap1.sum())
+        # algorithmic bytes: U row, one table row (hi + lo) per factor; with the gradient a second table row and the pmi
+        # gradient row per factor and given token, the pmi_w1 gradient row of each gap-1 one, and the ed / ped rows; the
+        # conditional row when asked for
+        self._timed('K13 pseudo_likelihood',
+                    lambda: (nv + n_nb) * V * 4.0 + ((n_nb + n_giv) * V * 8.0 + n_gap1 * V * 4.0 + 2 * nv * V * 4.0
+                                                     if want_grad else 0.0)
+                    + (nv * V * 4.0 if want_rows else 0.0),
+                    lambda: k.call('mlbp_pseudo_likelihood', ns, int(np.diff(corpus.var_off).max()), nv, c('var_off'),
+                                   c('pair_off'), c('pair_v0'), c('pair_v1'), c('pair_gap1'), c('var_label'), c('var_de'),
+                                   c('sp_off'), c('sp_en'), c('sp_feat'), c('sp_val'), c('giv_off'), c('giv_label'),
+                                   c('giv_gap1'), _p(U), _p(self.planes), V * ld, ld, V, self.scale_exp, _p(self.colsums),
+                                   _p(m.pmi), _p(m.w1), _p(m.edT), _p(m.pedT), ld, self._conditional_range_log2(corpus),
+                                   _p(logp_var), _p(top1), _p(rank), _p(g) if want_grad else None, _p(rows)))
+        grad, logp = torch.empty((ns, 9), dtype=torch.float64, device=dev), torch.empty(ns, dtype=torch.float64, device=dev)
+        k.call('mlbp_gradient_reduce', ns, c('var_off'), None, _p(g), _p(torch.zeros((1, 3), dtype=torch.float64, device=dev)),
+               None, None, c('var_label'), None, _p(m.pmi), _p(m.w1), ld, _p(logp_var), _p(grad), _p(logp))
+        self.launches += 2
+        if reduce_into is not None:
+            k.call('mlbp_batch_reduce', ns, _p(grad) if want_grad else None, _p(logp), nv, _p(rank), None, _p(reduce_into))
+            self.launches += 1
+        return grad, logp, logp_var, top1, rank, rows
 
     # ------------------------------------------------------------------ micro-batching
     def microbatches(self, corpus, sweeps, want_grad):

@@ -59,6 +59,10 @@ def parse(argv=None):
     opt.add_argument('--map_decode', dest='map_decode', default=False, action='store_true')
     # not a reference flag: also sample every sentence's joint guesses (Gibbs, Engine.sample): N burn-in and N kept sweeps, 4 chains
     opt.add_argument('--gibbs', dest='gibbs', type=int, default=None)
+    # not a reference flag: SGD on the pseudo-likelihood's exact gradient (Engine.pseudo_likelihood) instead of loopy BP's
+    opt.add_argument('--objective', dest='objective', choices=('lbp', 'pl'), default='lbp')
+    # not a reference flag: also report the pseudo-likelihood of the labels wherever BP's prediction statistics are reported
+    opt.add_argument('--pseudo_likelihood', dest='pseudo_likelihood', default=False, action='store_true')
     return opt.parse_args(argv)
 
 
@@ -206,7 +210,7 @@ def merge_parts(path, parts, spans):
 
 
 class SentenceLines(object):
-    """A one-line-per-sentence output file (.joint, .map, .gibbs): each rank writes the lines of its sentences to
+    """A one-line-per-sentence output file (.joint, .map, .gibbs, .pl): each rank writes the lines of its sentences to
     <path>.rank<r>.part and, after a barrier, rank 0 merges the parts in file order."""
 
     def __init__(self, path, rank, world):
@@ -240,7 +244,7 @@ GIBBS_CHAINS = 4
 
 
 def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None, out_path=None, joint=False, map_decode=False,
-            gibbs=0):
+            gibbs=0, pseudo=False):
     """train.py:308-338 batched and sharded over the torchrun ranks.  `units`: prediction_units(); `thetas`: domain ->
     (theta_ee, theta_ed) for the adaptation modes (else the engine's current theta is used).  The roots of every sentence are
     drawn from `rng` in unit order before the units are shared out, so a sentence gets the same roots on any number of ranks.
@@ -256,7 +260,10 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
     sentence's line index as its id; no draws from `rng`); one more result (sum over sentences of the Monte Carlo sum of log
     p(label), #rank == 0, largest across-chain standard error of a label probability), and with `out_path` the file
     <out_path>.gibbs, one line  sent_id TAB Gibbs log p(label) TAB standard errors TAB BP logp_var  (per token in position order)
-    per sentence in file order."""
+    per sentence in file order.
+    `pseudo`: every unit's pseudo-likelihood too (Engine.pseudo_likelihood; no draws from `rng`); one more result (sum over
+    sentences of the sum of log p(y_i | y_-i), #conditional arg-max == label), and with `out_path` the file <out_path>.pl, one
+    line  sent_id TAB log p(y_i | y_-i) TAB BP logp_var  (per token in position order)  per sentence in file order."""
     import torch
     from .engine import Corpus
     from .trainer import dist_info
@@ -265,8 +272,8 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
     corpora = [Corpus([sents[i] for i in idx]) for _, idx in units]
     roots = [draw_roots(c, 3, rng) for c in corpora]
     # per unit: sum logp, #rank == 0, < 26, < 50, variables, sum joint, MAP tokens right, MAP sentences right, Gibbs sum logp,
-    # Gibbs #rank == 0, largest Gibbs standard error
-    stats = np.zeros((len(units), 11))
+    # Gibbs #rank == 0, largest Gibbs standard error, pseudo-likelihood, pseudo #rank == 0
+    stats = np.zeros((len(units), 13))
     write = bool(out_path) and not qp
     if write:
         parts = [out_path + '.rank%d.part' % r for r in range(world)]
@@ -276,6 +283,7 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
     wj = SentenceLines(out_path + '.joint', rank, world) if (out_path and joint) else None
     wm = SentenceLines(out_path + '.map', rank, world) if (out_path and map_decode) else None
     wg = SentenceLines(out_path + '.gibbs', rank, world) if (out_path and gibbs) else None
+    wl = SentenceLines(out_path + '.pl', rank, world) if (out_path and pseudo) else None
     pinned = [None]
     cur = object()
     for u in range(rank, len(units), world):
@@ -321,6 +329,17 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
                     lo, hi = int(corpus.var_off[si]), int(corpus.var_off[si + 1])
                     cols = [' '.join('%r' % float(v) for v in a[lo:hi]) for a in (glv, se, blv)]
                     wg.write(i, '\t'.join([str(nodes[0]['sent_id'])] + cols) + '\n')
+        if pseudo:
+            rp = engine.pseudo_likelihood(corpus, want_grad=False)
+            plv, prk = rp.logp_var.cpu().numpy(), rp.rank.cpu().numpy()
+            stats[u, 11:13] = (float(rp.logp.sum().item()), int((prk == 0).sum()))
+            if wl:
+                blv = r.logp_var.cpu().numpy()
+                for si, i in enumerate(idx):
+                    nodes = sorted(raw[i]['current_sent'], key=lambda n: int(n['position']))
+                    lo, hi = int(corpus.var_off[si]), int(corpus.var_off[si + 1])
+                    cols = [' '.join('%r' % float(v) for v in a[lo:hi]) for a in (plv, blv)]
+                    wl.write(i, '\t'.join([str(nodes[0]['sent_id'])] + cols) + '\n')
         if not write:
             continue
         text, toff = dist_text(engine, r.beliefs, pinned)
@@ -378,11 +397,11 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
                     where[i] = (rr, po, pl, do, dl)
             merge_parts(out_path, parts, [(w[0], w[1], w[2]) for w in where])
             merge_parts(out_path + '.dist', dparts, [(w[0], w[3], w[4]) for w in where])
-    for w in (wj, wm, wg):
+    for w in (wj, wm, wg, wl):
         if w:
             w.merge(len(sents))
     sums = []
-    for col in (0, 5, 8):
+    for col in (0, 5, 8, 11):
         total, k = 0.0, 0
         while k < len(units):                                   # one partial sum per domain, as the single-process loop
             part, d = 0.0, units[k][0]
@@ -399,6 +418,8 @@ def predict(engine, units, sents, raw, en_domain, options, rng, qp, thetas=None,
         out += (tuple(int(x) for x in stats[:, 6:8].sum(axis=0)),)
     if gibbs:
         out += ((sums[2], int(stats[:, 9].sum()), float(stats[:, 10].max()) if len(units) else 0.0),)
+    if pseudo:
+        out += ((sums[3], int(stats[:, 12].sum())),)
     return out
 
 
@@ -415,6 +436,12 @@ def print_gibbs(prefix, res, n_lines, n_tokens):
     print(prefix + 'prediction Gibbs probs:', res[0] / float(n_lines))
     print(prefix + 'prediction Gibbs Prec at 0:', '%0.2f' % (float(100 * res[1]) / float(max(n_tokens, 1))), 'total:', n_tokens)
     print(prefix + 'prediction Gibbs max standard error:', res[2])
+
+
+def print_pl(prefix, res, n_lines, n_tokens):
+    """the two --pseudo_likelihood lines: the exact-conditional counterparts of `prediction probs:` and of `Prec at 0:`"""
+    print(prefix + 'prediction pseudo log-likelihood:', res[0] / float(n_lines))
+    print(prefix + 'prediction pseudo Prec at 0:', '%0.2f' % (float(100 * res[1]) / float(max(n_tokens, 1))), 'total:', n_tokens)
 
 
 def main(argv=None):
@@ -435,6 +462,11 @@ def main(argv=None):
         sys.stderr.write('--gibbs N needs N >= 1 (burn-in and kept sweeps per chain)\n')
         return 1
     adapt = options.user_adapt or options.experience_adapt
+    if options.objective == 'pl' and (adapt or options.use_approx_inference or options.use_approx_beliefs):
+        sys.stderr.write('--objective pl trains the base theta on exact conditionals: it does not combine with --user_adapt, '
+                         '--experience_adapt, --use_approx_inference or --use_approx_beliefs\n')
+        return 1
+    pl = options.objective == 'pl'
     import os
     import torch
     from .engine import Corpus, Engine
@@ -518,7 +550,7 @@ def main(argv=None):
         return 0
     if mode == 'training':
         mb = options.minibatch or (4 if options.cpus.strip() == '' else int(options.cpus))     # train_mp.py:493
-        tr = Trainer(engine, reg_param=float(options.reg_param), N=len(train_lines))
+        tr = Trainer(engine, reg_param=float(options.reg_param), N=len(train_lines), objective=options.objective)
         tr.theta_ee, tr.theta_ed = theta_ee.reshape(-1).copy(), theta_ed.reshape(-1).copy()
         sents = lower(train_lines, options, en2id, de2id)
         order = list(range(len(sents)))
@@ -529,12 +561,12 @@ def main(argv=None):
             for lo in range(0, len(order), mb):
                 batch = [sents[i] for i in order[lo:lo + mb]][rank::world]
                 corpus = Corpus(batch)                  # an empty shard contributes a zero vector to the all-reduce
-                red = tr.step(corpus, draw_roots(corpus, 3, rng), lr, **approx_kw)
+                red = tr.step(corpus, None if pl else draw_roots(corpus, 3, rng), lr, **approx_kw)
                 logp += tr.apply(red, lr)[9]
             print('\nepoch:', epoch)
             print(f_en_en_names, tr.theta_ee)
             print(f_en_de_names, tr.theta_ed)
-            print('\ntrain prediction probs:', logp / float(len(sents)))
+            print('\ntrain pseudo log-likelihood:' if pl else '\ntrain prediction probs:', logp / float(len(sents)))
             if rank == 0 and options.save_params_file:
                 save_params(codecs.open(options.save_params_file + '.iter' + str(epoch), 'w', 'utf8'), tr.theta_ee.reshape(1, -1),
                             tr.theta_ed.reshape(1, -1), f_en_en_names, f_en_de_names, {})
@@ -544,7 +576,7 @@ def main(argv=None):
                 tune_sents = lower(tune_lines, options, en2id, de2id)
                 res = predict(engine, prediction_units(len(tune_sents)), tune_sents, [json.loads(l) for l in tune_lines],
                               en_domain, options, rng, True, joint=options.joint_likelihood, map_decode=options.map_decode,
-                              gibbs=options.gibbs or 0)
+                              gibbs=options.gibbs or 0, pseudo=options.pseudo_likelihood)
                 lp, (p0, p25, p50, tot) = res[:2]
                 if rank == 0:
                     print('\ntune prediction probs:', lp / float(len(tune_lines)))
@@ -555,7 +587,10 @@ def main(argv=None):
                     if options.map_decode:
                         print_map('tune ', res[2 + bool(options.joint_likelihood)], tot, len(tune_sents))
                     if options.gibbs:
-                        print_gibbs('tune ', res[-1], len(tune_lines), tot)
+                        print_gibbs('tune ', res[2 + bool(options.joint_likelihood) + bool(options.map_decode)], len(tune_lines),
+                                    tot)
+                    if options.pseudo_likelihood:
+                        print_pl('tune ', res[-1], len(tune_lines), tot)
         print('\ntheta final:', tr.theta_ee, tr.theta_ed)
         if rank == 0 and options.save_params_file:
             save_params(codecs.open(options.save_params_file, 'w', 'utf8'), tr.theta_ee.reshape(1, -1), tr.theta_ed.reshape(1, -1),
@@ -574,7 +609,7 @@ def main(argv=None):
         thetas, units = None, prediction_units(len(all_sents))
     res = predict(engine, units, all_sents, raw, en_domain, options, rng, options.quick_predict, thetas,
                   options.save_predictions_file, joint=options.joint_likelihood, map_decode=options.map_decode,
-                  gibbs=options.gibbs or 0)
+                  gibbs=options.gibbs or 0, pseudo=options.pseudo_likelihood)
     lp, (p0, p25, p50, tot) = res[:2]
     if rank == 0:
         print('\nprediction probs:', lp / float(len(train_lines)))
@@ -585,7 +620,9 @@ def main(argv=None):
         if options.map_decode:
             print_map('', res[2 + bool(options.joint_likelihood)], tot, len(all_sents))
         if options.gibbs:
-            print_gibbs('', res[-1], len(train_lines), tot)
+            print_gibbs('', res[2 + bool(options.joint_likelihood) + bool(options.map_decode)], len(train_lines), tot)
+        if options.pseudo_likelihood:
+            print_pl('', res[-1], len(train_lines), tot)
     if torch.cuda.is_available():
         torch.cuda.synchronize()
     return 0

@@ -26,8 +26,13 @@ def dist_info():
 
 
 class Trainer(object):
-    def __init__(self, engine, reg_param=0.2, N=None, sweeps=3, init_lr=0.1):
+    def __init__(self, engine, reg_param=0.2, N=None, sweeps=3, init_lr=0.1, objective='lbp'):
+        if objective not in ('lbp', 'pl'):
+            raise ValueError("objective must be 'lbp' (the reference's loopy-BP gradient) or 'pl' (the pseudo-likelihood)")
         self.engine = engine
+        # 'pl': step() follows the exact gradient of the pseudo-likelihood (Engine.pseudo_likelihood, K13) instead of BP's;
+        # the 16-vector, the all-reduce and apply() are the same, eval_step() stays BP prediction
+        self.objective = objective
         self.reg_param = float(reg_param)
         self.N = N                                  # len(training_instances), train.py:619 (reg = reg_param / N, :158)
         self.sweeps = sweeps
@@ -53,13 +58,22 @@ class Trainer(object):
 
     def _reduce(self, parts_or_corpus, roots, want_grad, all_reduce, next_roots=None, **kw):
         eng = self.engine
+        pl = want_grad and self.objective == 'pl'
+        if pl and not isinstance(parts_or_corpus, Corpus):
+            raise ValueError("objective='pl' steps take a Corpus: prepared BP parts carry BP's micro-batching, not K13's")
+        if pl and any(kw.values()):
+            raise ValueError("objective='pl' steps run exact conditionals: BP options (%s) do not apply"
+                             % ', '.join(k for k, v in kw.items() if v))
         eng.set_theta(self.theta_ee, self.theta_ed, with_grad=want_grad)
         if self._red is None:
             self._red = torch.zeros(16, dtype=torch.float64, device=eng.device)
         red = self._red                                        # the all-reduce buffer: every micro-batch is added on the device
         eng.k.call('mlbp_zero_words', ctypes.c_void_p(red.data_ptr()), 32)
-        fn = eng.run_many if isinstance(parts_or_corpus, Corpus) else eng.run_prepared
-        fn(parts_or_corpus, roots, self.sweeps, want_grad, True, reduce_into=red, collect=False, **kw)
+        if pl:                                                 # no roots: the pseudo-likelihood has no schedule
+            eng.pseudo_likelihood(parts_or_corpus, want_grad=True, reduce_into=red)
+        else:
+            fn = eng.run_many if isinstance(parts_or_corpus, Corpus) else eng.run_prepared
+            fn(parts_or_corpus, roots, self.sweeps, want_grad, True, reduce_into=red, collect=False, **kw)
         if next_roots is not None and not isinstance(parts_or_corpus, Corpus) and parts_or_corpus:
             lo, hi, c = parts_or_corpus[0]                          # everything of this step is enqueued: the host is free
             eng.precompile(c, np.ascontiguousarray(next_roots, dtype=np.int32)[lo:hi], self.sweeps, want_grad, True,
